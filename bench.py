@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- MPI frames/s (96 planes, 1024^2) on N B200s, with roofline, end-to-end, CPU-baseline and config legs.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Headline workload (BASELINE.json configs[2], "FFHQ1024"): per GPU a batch of 4 MPIs, 96 planes, 1024^2 textures, one
@@ -39,6 +39,7 @@ N_PLANES, RES, BATCH = 96, 1024, 4
 WORKLOAD = "FFHQ1024: 96 planes, 1024^2 textures and views, 4 MPIs x 1 view per GPU, forward render"
 METRIC = "MPI frames/s (96 planes, 1024^2)"
 VIDEO_VIEWS = 120
+DUMP_MAX_BYTES = 64 * 10**6       # --dump-outputs: the headline's 4 x 1024^2 frames (67 MB) are sampled to fit
 
 
 def algorithmic_bytes_fwd(n, ht, wt, h, w):
@@ -609,12 +610,14 @@ def leg_headline(job, args, NP, R, B):
     kernel_ms = sum(be.elapsed_ms(a, b) for a, b in kev) / args.steps
     total_ms, kernel_ms = job.max_over_ranks([total_ms, kernel_ms])
     ms_per_step = total_ms / args.steps
-    # device-resident result of the last step, for the e2e cross-check
+    # device-resident result of the last step, for the e2e cross-check; `frames` = every rank's frames after the all-gather
     if gather is not None:
         mine = gather.frames[rank * B:(rank + 1) * B]
         res_color, res_depth = mine[:, :3], mine[:, 3:]
+        frames = gather.frames
     else:
         res_color, res_depth = color, depth
+        frames = frames_all
     peak, peak_src = measured_peak()
     alg = algorithmic_bytes_fwd(NP, R, R, R, R) * B
     achieved = alg / (kernel_ms * 1e-3) / 1e9
@@ -631,7 +634,33 @@ def leg_headline(job, args, NP, R, B):
                 "algorithmic_bytes_per_launch": alg, "peak_source": peak_src}
     out = {"frames_per_s": world * B / (ms_per_step * 1e-3), "ms_per_step": ms_per_step, "clocks": clocks, "launches": launches[0],
            "roofline": roofline, "gather_mode": gather_mode}
-    return out, {"case": case, "color": res_color, "depth": res_depth, "gather": gather}
+    return out, {"case": case, "color": res_color, "depth": res_depth, "gather": gather, "frames": frames}
+
+
+def dump_outputs(dirname, color, depth, max_bytes=DUMP_MAX_BYTES):
+    """Writes a headline step's frames as float32 .npy files, so that two builds run with the same arguments (hence the same
+    seeded inputs) can be compared output for output.  Pixels p = (view * H + y) * W + x of color [V,3,H,W] and depth
+    [V,1,H,W] go to color.npy [P,3], depth.npy [P] and pixel_index.npy [P] (p as float64).  When all pixels would exceed
+    max_bytes, P is a fixed sample (seed 0, sorted) of as many pixels as fit.  Returns {name: shape}."""
+    import numpy as np
+    import torch
+    V, _, H, W = color.shape
+    n_pix = V * H * W
+    per_pixel = 3 * 4 + 4 + 8
+    budget = max_bytes - 3 * 1024                  # room for the three .npy headers
+    if n_pix * per_pixel <= budget:
+        idx = np.arange(n_pix)
+    else:
+        idx = np.sort(np.random.default_rng(0).choice(n_pix, budget // per_pixel, replace=False))
+    sel = torch.from_numpy(idx).to(color.device)
+    out = {"color": color.permute(0, 2, 3, 1).reshape(n_pix, 3).index_select(0, sel),
+           "depth": depth.reshape(n_pix).index_select(0, sel)}
+    out = {k: v.float().cpu().numpy() for k, v in out.items()}
+    out["pixel_index"] = idx.astype(np.float64)
+    os.makedirs(dirname, exist_ok=True)
+    for k, v in out.items():
+        np.save(os.path.join(dirname, k + ".npy"), v)
+    return {k: list(v.shape) for k, v in out.items()}
 
 
 def leg_train(job, case, steps, NP, R, B):
@@ -884,8 +913,14 @@ def _main(argv, out):
     ap.add_argument("--planes", type=int, default=N_PLANES)
     ap.add_argument("--res", type=int, default=RES)
     ap.add_argument("--batch", type=int, default=BATCH)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the frames of the last one (colour and depth "
+                    "of every view, float32 .npy; a fixed sample of pixels beyond 64 MB) to DIR")
     ap.add_argument("--fake", action="store_true", help=argparse.SUPPRESS)     # tests/test_bench_flow.py only
     args = ap.parse_args(argv)
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     if args.impl == "reference":
         return run_reference_arm(args, out)
     args.warmup = max(args.warmup, 3)
@@ -900,6 +935,11 @@ def _main(argv, out):
     NP, R, B = be.sizes(args.planes, args.res, args.batch)
 
     head, state = leg_headline(job, args, NP, R, B)
+    if args.dump_outputs and rank == 0:
+        frames = state["frames"]
+        color, depth = (state["color"], state["depth"]) if frames is None else (frames[:, :3], frames[:, 3:])
+        written = dump_outputs(args.dump_outputs, color, depth)
+        print(f"[bench] wrote {written} to {args.dump_outputs}", file=sys.stderr)
     train = None
     if not args.no_train_step:
         train = leg_train(job, state["case"], max(3, min(args.steps, 5)), NP, R, B)

@@ -57,6 +57,48 @@ def test_default_command_line_runs_every_leg(world, no_symm):
         assert "fused" in par
 
 
+@pytest.mark.parametrize("world", [1, 2])
+def test_dump_outputs_writes_the_last_timed_step_reproducibly(world, tmp_path):
+    """--dump-outputs DIR: the headline's frames (every rank's, after the all-gather) as float32 .npy, the same from run to run;
+    --steps sets the number of timed launches."""
+    import numpy as np
+    runs = []
+    for i in range(2 if world == 1 else 1):
+        d = tmp_path / f"run{i}"
+        line = _run(world, extra_args=("--steps", "5", "--dump-outputs", str(d)))
+        assert line["steps"] == 5 and line["gpu_launches"] == 5
+        runs.append({k: np.load(d / f"{k}.npy") for k in ("color", "depth", "pixel_index")})
+    n_pix = world * 2 * 16 * 16                                       # FakeBackend.sizes: 2 MPIs x 1 view, 16^2, per rank
+    got = runs[0]
+    assert got["color"].shape == (n_pix, 3) and got["depth"].shape == (n_pix,)
+    assert got["color"].dtype == np.float32 and got["depth"].dtype == np.float32
+    assert np.array_equal(got["pixel_index"], np.arange(n_pix, dtype=np.float64))
+    assert np.all(np.isfinite(got["color"])) and np.all(got["depth"] > 0)
+    for other in runs[1:]:
+        assert all(np.array_equal(got[k], other[k]) for k in got)
+
+
+def test_dump_outputs_samples_a_fixed_set_of_pixels_beyond_the_cap(tmp_path):
+    import numpy as np
+    import torch
+    import bench
+    gen = torch.Generator().manual_seed(3)
+    color, depth = torch.rand(3, 3, 20, 24, generator=gen), torch.rand(3, 1, 20, 24, generator=gen)
+    cap = 3 * 1024 + 1000 * 24                                        # headers + 1000 of the 1440 pixels
+    shapes = bench.dump_outputs(str(tmp_path / "a"), color, depth, max_bytes=cap)
+    assert shapes == {"color": [1000, 3], "depth": [1000], "pixel_index": [1000]}
+    assert sum(f.stat().st_size for f in (tmp_path / "a").iterdir()) <= cap
+    idx = np.load(tmp_path / "a" / "pixel_index.npy")
+    p = idx.astype(np.int64)
+    assert np.array_equal(p, np.unique(p)) and p.max() < 1440
+    v, y, x = p // (20 * 24), p // 24 % 20, p % 24
+    np.testing.assert_array_equal(np.load(tmp_path / "a" / "color.npy"), color.numpy()[v, :, y, x])
+    np.testing.assert_array_equal(np.load(tmp_path / "a" / "depth.npy"), depth.numpy()[v, 0, y, x])
+    bench.dump_outputs(str(tmp_path / "b"), color * 2, depth, max_bytes=cap)
+    assert np.array_equal(np.load(tmp_path / "b" / "pixel_index.npy"), idx)          # the sample does not depend on the data
+    assert bench.DUMP_MAX_BYTES <= 64 * 10**6
+
+
 def test_reference_arm_only_rank0_prints_and_others_exit_zero():
     env = dict(os.environ, RANK="1", LOCAL_RANK="1", WORLD_SIZE="2")
     r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--gpus", "2"], env=env,

@@ -1,35 +1,63 @@
 """Drop-in boundary: the host-side mirrors must accept exactly what the reference's callers pass (SURVEY.md 8b).
-Runs only where /root/reference exists (the build container); the GPU box skips it."""
+The reference's signatures and the MPI construction + call its MPIRenderer.render makes were recorded from the unmodified
+reference (tests/golden/reference_signatures.json, tests/golden/reference_mpi_call.npz, oracle/make_golden_interface.py)."""
 import inspect
+import json
+import os
 
+import numpy as np
 import pytest
+import torch
 
-import ref_shim
-
-pytestmark = pytest.mark.skipif(not ref_shim.reference_available(), reason="reference not mounted")
+from conftest import GOLDEN
 
 
 def _params(fn):
-    return [(n, p.kind, p.default) for n, p in inspect.signature(fn).parameters.items() if n != "self"]
+    """The rows oracle/make_golden_interface.py recorded: (name, kind, repr(default)) without self."""
+    return [[n, p.kind.name, repr(p.default)] for n, p in inspect.signature(fn).parameters.items() if n != "self"]
+
+
+def _reference_signatures():
+    with open(os.path.join(GOLDEN, "reference_signatures.json")) as f:
+        return json.load(f)
+
+
+def _decode_kwargs(z, prefix):
+    """Inverse of make_golden_interface.encode_kwargs: the keyword arguments in the order the reference passed them."""
+    kw = {}
+    for name in z[prefix + "order"]:
+        name = str(name)
+        if f"{prefix}none/{name}" in z.files:
+            kw[name] = None
+        elif f"{prefix}t/{name}" in z.files:
+            kw[name] = torch.from_numpy(z[f"{prefix}t/{name}"])
+        elif f"{prefix}a/{name}" in z.files:
+            kw[name] = z[f"{prefix}a/{name}"]
+        elif f"{prefix}s/{name}" in z.files:
+            kw[name] = z[f"{prefix}s/{name}"].item()
+        else:
+            n = sum(1 for k in z.files if k.startswith(f"{prefix}l/{name}/"))
+            assert n > 0, name
+            kw[name] = [torch.from_numpy(z[f"{prefix}l/{name}/{i}"]) for i in range(n)]
+    return kw
 
 
 def test_mpi_signatures():
-    ref_mpi, _ = ref_shim.import_reference()
+    ref = _reference_signatures()["MPI"]
     import ml_gmpi_b200 as g
-    ours, theirs = _params(g.MPI.forward), _params(ref_mpi.MPI.forward)
-    assert ours == theirs                                            # keyword-only, same names, same defaults
-    assert _params(g.MPI.check_shapes) == _params(ref_mpi.MPI.check_shapes)
-    init_ref = _params(ref_mpi.MPI.__init__)
+    assert _params(g.MPI.forward) == ref["forward"]                  # keyword-only, same names, same defaults
+    assert _params(g.MPI.check_shapes) == ref["check_shapes"]
+    init_ref = ref["__init__"]
     init_ours = _params(g.MPI.__init__)
     assert init_ours[: len(init_ref)] == init_ref                    # ours adds the optional `validate` after align_corners
 
 
 def test_renderer_signatures():
-    _, ref_r = ref_shim.import_reference()
+    ref = _reference_signatures()["MPIRenderer"]
     from ml_gmpi_b200.renderer import MPIRenderer
     for name in ("render", "sample_cam_poses", "set_cam", "compute_mpi_spatial_volume"):
-        assert _params(getattr(MPIRenderer, name)) == _params(getattr(ref_r.MPIRenderer, name)), name
-    ref_init = _params(ref_r.MPIRenderer.__init__)
+        assert _params(getattr(MPIRenderer, name)) == ref[name], name
+    ref_init = ref["__init__"]
     ours_init = _params(MPIRenderer.__init__)
     assert ours_init[: len(ref_init)] == ref_init                    # ours adds the optional `validate`
 
@@ -43,29 +71,22 @@ def test_reference_call_site_binds():
 
 
 def test_unmodified_reference_renderer_drives_the_drop_in():
-    """INTEGRATION.md's patch, executed: `gmpi.core.mpi_renderer.MPI = ml_gmpi_b200.MPI`, then the UNMODIFIED reference
-    MPIRenderer is constructed (mpi_renderer.py:47 instantiates our class) and `render` is called with real tensors.  The call
-    must get through the reference's own pose sampling / ray generation (mpi_renderer.py:418-449) and our check_shapes with the
-    reference's real argument list (mpi_renderer.py:451-461), and stop exactly at the "CUDA devices only" check -- there is no
-    GPU in the build container and no CPU fallback by design."""
-    import torch
+    """INTEGRATION.md's patch (`gmpi.core.mpi_renderer.MPI = ml_gmpi_b200.MPI`), replayed: the unmodified reference
+    MPIRenderer constructs MPI (mpi_renderer.py:47) and, inside `render`, calls it with the tensors its own pose sampling and
+    ray generation produced (mpi_renderer.py:418-461).  Both were recorded; replayed against our class, the construction must
+    take the reference's keywords and the call must get through our check_shapes and stop exactly at the "CUDA devices only"
+    check -- the recorded tensors live on the CPU and there is no CPU fallback by design."""
     import ml_gmpi_b200 as g
-    _, ref_r = ref_shim.import_reference()
-    old = ref_r.MPI
-    ref_r.MPI = g.MPI
-    try:
-        r = ref_r.MPIRenderer(n_mpi_planes=4, plane_min_d=0.95, plane_max_d=1.12, plan_spatial_enlarge_factor=1.001,
-                              plane_distances_sample_method="inverse", cam_fov=12.6, sphere_center_z=1.0, sphere_r=1.0,
-                              horizontal_mean=0.0, horizontal_std=0.289, vertical_mean=0.0, vertical_std=0.127,
-                              cam_pose_n_truncated_stds=2, cam_sample_method="truncated_gaussian", mpi_align_corners=True,
-                              use_confined_volume=True, device=torch.device("cpu"))
-        assert isinstance(r.mpi, g.MPI) and r.mpi._align_corners is True
-        rgba = torch.rand(2, 4, 4, 16, 16)
-        with pytest.raises(RuntimeError, match="CUDA devices only"):
-            r.render(rgba, 16, 16, given_yaws=torch.zeros(2, 1), given_pitches=torch.zeros(2, 1))
-        # a malformed MPI is rejected by OUR check_shapes with the reference's message before any device work
-        with pytest.raises(AssertionError, match="Expected rgba to be of shape"):
-            r.mpi(batch_rgba=torch.rand(2, 4, 3, 16, 16), batch_dhw=torch.rand(2, 4, 3), batch_ray_dir=[torch.rand(1, 3, 8, 8)] * 2,
-                  batch_eye_pos=[torch.rand(1, 3)] * 2, batch_z_dir=[torch.rand(1, 3)] * 2, separate_background=None)
-    finally:
-        ref_r.MPI = old
+    z = np.load(os.path.join(GOLDEN, "reference_mpi_call.npz"))
+    init_kw, call_kw = _decode_kwargs(z, "init/"), _decode_kwargs(z, "call/")
+    assert list(call_kw) == ["batch_rgba", "batch_dhw", "batch_ray_dir", "batch_eye_pos", "batch_z_dir", "separate_background",
+                             "assert_not_out_of_last_plane", "c2w_mat", "sphere_c"]
+    mpi = g.MPI(**init_kw)
+    assert mpi._align_corners is True
+    assert call_kw["batch_rgba"].shape == (2, 4, 4, 16, 16) and len(call_kw["batch_ray_dir"]) == 2
+    with pytest.raises(RuntimeError, match="CUDA devices only"):
+        mpi(**call_kw)
+    # a malformed MPI is rejected by OUR check_shapes with the reference's message before any device work
+    with pytest.raises(AssertionError, match="Expected rgba to be of shape"):
+        mpi(batch_rgba=torch.rand(2, 4, 3, 16, 16), batch_dhw=torch.rand(2, 4, 3), batch_ray_dir=[torch.rand(1, 3, 8, 8)] * 2,
+            batch_eye_pos=[torch.rand(1, 3)] * 2, batch_z_dir=[torch.rand(1, 3)] * 2, separate_background=None)

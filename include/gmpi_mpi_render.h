@@ -175,6 +175,21 @@ int gmpi_mpi_render_bwd_saved(const float* rgba, const int32_t* view2mpi, const 
  *   transmittance [V,N,H,W]                      training forward: saved for gmpi_mpi_render_bwd_ex
  *   backward: g_color [V,3,H,W], g_depth (nullable), and g_rgba [M,N,4,Ht,Wt]  or  g_rgb [M,3,Ht,Wt] (+ g_bg_rgb) + g_alpha
  *             [M,N,1,Ht,Wt]; zeroed by the callee with GMPI_ZERO_GRAD, else accumulated into
+ *   stop_transmittance  tau in [0, 1): early ray termination of the INFERENCE forward (0 = off, the default).
+ *               A pixel's colour and depth may drop the contributions of the planes behind the point where its transmittance
+ *               T = prod_{j<i}(1 - alpha_j) is already below tau.  Hence every output lies in [full - tau * max(value), full]
+ *               (colour in [0,1], and depth; plus fp32 rounding; twice that for 2c-1 colour), a pixel whose T stays >= tau up
+ *               to the last plane is bit-identical to the tau = 0 render, and tau = 0 is bit-identical to a descriptor without
+ *               the field.  Deterministic: the same inputs give the same bytes and the same skip count.  The staged kernels
+ *               stop a 64x30 tile once all its pixels are below tau (a few planes later: the planes already in flight are
+ *               composited); the direct kernel stops each pixel on its own.  Rejected (GMPI_ERR_INVALID_ARGUMENT, before any
+ *               CUDA call): tau NaN, < 0 or >= 1; tau > 0 together with `transmittance` (the training forward saves every T);
+ *               tau > 0 in gmpi_mpi_render_bwd_ex (gradients stay exact).
+ *   skipped_pixel_planes  nullable uint64 [1], device memory (host memory for gmpi_mpi_render_host_ex): accumulated into, the
+ *               number of (pixel, plane) pairs not composited because of stop_transmittance.  Not zeroed by the callee.
+ *   The last two fields were appended without changing GMPI_ABI_VERSION: struct_bytes = offsetof(gmpi_render_desc,
+ *   stop_transmittance), the size of the descriptor before them, is still accepted and means both fields absent (tau = 0).
+ *   A caller that sets them against an older library gets the struct_bytes error, never a silently exact render.
  */
 typedef struct gmpi_render_desc {
     uint32_t struct_bytes;
@@ -207,6 +222,8 @@ typedef struct gmpi_render_desc {
     float* g_alpha;
     uint32_t* flags;
     void* stream;
+    float stop_transmittance;
+    uint64_t* skipped_pixel_planes;
 } gmpi_render_desc;
 
 /* cudaMemsetAsync(ptr, 0, bytes) on `stream`, for callers that accumulate into their own buffers (no GMPI_ZERO_GRAD).  Note that a

@@ -43,7 +43,12 @@ class RenderDesc(ctypes.Structure):
                 ("depth_near", ctypes.c_float), ("depth_range", ctypes.c_float)] + \
                [(n, ctypes.c_void_p) for n in ("rgba", "rgb", "alpha", "bg_rgb", "view2mpi", "dhw", "ray_dir", "eye", "z_dir", "cam",
                                                "color", "depth", "transmittance", "peer_frames", "video_rgb", "video_depth",
-                                               "g_color", "g_depth", "g_rgba", "g_rgb", "g_bg_rgb", "g_alpha", "flags", "stream")]
+                                               "g_color", "g_depth", "g_rgba", "g_rgb", "g_bg_rgb", "g_alpha", "flags", "stream")] + \
+               [("stop_transmittance", ctypes.c_float), ("skipped_pixel_planes", ctypes.c_void_p)]     # appended (early termination)
+
+
+# struct_bytes of the descriptor before the early-termination fields: still accepted, the fields then read as absent
+DESC_BYTES_WITHOUT_STOP = RenderDesc.stop_transmittance.offset
 
 
 def make_desc(**kw) -> RenderDesc:

@@ -56,6 +56,10 @@ struct RenderParams {
     unsigned long long zero_slab16;
     unsigned* zero_flags;
     int zero_rate;
+    // inference forward (opt-in): early ray termination.  A pixel may drop the planes behind the point where its transmittance
+    // fell below stop_transmittance (0 = off); skipped (nullable, device) accumulates the pixel-planes not composited.
+    float stop_transmittance;
+    unsigned long long* skipped;
 };
 
 // The four channel slabs (Ht*Wt floats each) of one (MPI, plane): expanded rgba or the generator's factored form.

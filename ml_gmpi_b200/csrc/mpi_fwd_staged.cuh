@@ -68,10 +68,18 @@ struct __align__(16) StageMeta {
                            // down) - cx is floor(x) relative to the box
     int rows2;             // staged rows - 2: a footprint with north-west tap (rx, ry) fits iff 0<=rx<=bw-2, 0<=ry<=rows-2
     int sel;               // bits 0-7 staged width (row pitch = 4*bw floats), bits 8-9 mode (0 staged, 1 nothing under the
-                           // tile, 2 sample from global), bits 16-20 width class for the packed fast body, ONE-HOT (a chain of
-                           // single-bit tests, most frequent first, is shorter than a jump table), or 0 (not usable: mode != 0,
-                           // or plane constants outside the exact-division range)
+                           // tile, 2 sample from global, 3 end of tile: early ray termination, see kModeEnd), bits 16-20 width
+                           // class for the packed fast body, ONE-HOT (a chain of single-bit tests, most frequent first, is
+                           // shorter than a jump table), or 0 (not usable: mode != 0, or plane constants outside the
+                           // exact-division range)
 };
+// Early ray termination (the kCut forward, inference only): after every plane each active consumer warp ORs "some pixel of mine
+// still has T >= stop_transmittance" into the stage's vote word.  Before the producer reuses a stage it has waited for every
+// consumer's release of the plane kStages earlier; if that plane's vote is zero the whole tile is below the threshold, and
+// instead of the next plane the producer publishes a header with this mode (no copies, no tx bytes).  Consumers finish the
+// planes in flight, see it in the generic body, release the stage and go to the epilogue.  The producer alone decides, so the
+// ring stays in lockstep and the result does not depend on timing.
+constexpr int kModeEnd = 3;
 
 // ---- packed dual-fp32 arithmetic (sm_100 FFMA2/FADD2/FMUL2): one issue slot for two pixels, IEEE rn per element ----
 typedef float2 f2;
@@ -295,15 +303,21 @@ struct TileWalk {
     }
 };
 
-// A consumer warp without a single row inside the image: hand every stage of this tile straight back to the producer.
-__device__ __forceinline__ void consumer_idle_tile(uint64_t* s_full, uint64_t* s_empty, int N, int lane, int& c_stage, uint32_t& c_phase) {
+// A consumer warp without a single row inside the image: hand every stage of this tile straight back to the producer (kCut: up to
+// and including an end-of-tile header; such a warp does not vote).
+template <bool kCut = false>
+__device__ __forceinline__ void consumer_idle_tile(uint64_t* s_full, uint64_t* s_empty, int N, int lane, int& c_stage, uint32_t& c_phase,
+                                                   const StageMeta* s_meta = nullptr) {
     for (int i = 0; i < N; ++i) {
         const int s = c_stage;
         const uint32_t ph = c_phase;
         if (++c_stage == kStages) { c_stage = 0; c_phase ^= 1u; }
         mbar_wait(&s_full[s], ph);
+        bool end = false;
+        if constexpr (kCut) end = ((s_meta[s].sel >> 8) & 3) == kModeEnd;
         __syncwarp();
         mbar_arrive_if(&s_empty[s], lane == 0);
+        if (end) break;
     }
 }
 
@@ -357,9 +371,12 @@ struct NoPacer { static constexpr bool kActive = false; };      // the forward's
 // Pacer: an optional side job of the producer warp (the backward's gradient zeroing): before_tile(mpi) ahead of a tile's first
 // copy; new_stage() then chunk() between the polls of the wait for a free ring stage (chunk() returns false when there is nothing
 // to do); at_end() after the last tile.
-template <bool kAlignCorners, class Ring, bool kFact, class Pacer>
+// kCut (forward only): early ray termination, see kModeEnd.  s_vote[kStages] are the stages' vote words; `skipped` (nullable)
+// accumulates the pixel-planes of the tiles it cuts short.
+template <bool kAlignCorners, class Ring, bool kFact, class Pacer, bool kCut = false>
 __device__ __forceinline__ void staged_producer(const RenderParams& p, const TmaMaps& maps, float* s_buf, StageMeta* s_meta,
-                                            uint64_t* s_full, uint64_t* s_empty, const TileWalk* s_walk, int lane, Pacer& pacer) {
+                                            uint64_t* s_full, uint64_t* s_empty, const TileWalk* s_walk, int lane, Pacer& pacer,
+                                            uint32_t* s_vote = nullptr, unsigned long long* skipped = nullptr) {
     constexpr bool kReverse = Ring::kReverse;
     constexpr int kStride = Ring::kStride;      // floats per ring stage
     constexpr int kTileH = Ring::kTileRows, kStages = Ring::kRingStages, kMaxBH = Ring::kBoxMaxH, kStageFloats = Ring::kPlaneFloats;
@@ -422,6 +439,27 @@ __device__ __forceinline__ void staged_producer(const RenderParams& p, const Tma
                 mbar_wait_sleep(&s_empty[s], ph ^ 1);
             } else {
                 mbar_wait(&s_empty[s], ph ^ 1);
+            }
+            if constexpr (kCut) {
+                // every consumer has released plane ii - kStages of this tile, so its vote is complete (lane 0 reads it: the
+                // decision must be warp-uniform, and lane 0 clears the word below)
+                const uint32_t vote = __shfl_sync(0xffffffffu, lane == 0 ? *(volatile uint32_t*)&s_vote[s] : 0u, 0);
+                if (ii >= kStages && vote == 0) {
+                    if (lane == 0) {
+                        StageMeta mt;
+                        mt.cx = mt.cy = mt.rows2 = 0;
+                        mt.sel = kModeEnd << 8;
+                        s_meta[s] = mt;
+                        mbar_arrive(&s_full[s]);
+                        if (skipped) {
+                            const int tile_pix = min(kTileW, p.W - px0) * min(kTileH, p.H - py0);
+                            atomicAdd(skipped, (unsigned long long)(N - ii) * (unsigned long long)tile_pix);
+                        }
+                    }
+                    __syncwarp();
+                    break;
+                }
+                if (lane == 0) s_vote[s] = 0u;      // published below with the header (the arrive releases both)
             }
             if (lane == 0) {
                 StageMeta mt;
@@ -524,9 +562,13 @@ __device__ __forceinline__ void store_tile_pixels(const RenderParams& p, int v, 
 template <bool kFactored>
 using FwdRingFor = typename std::conditional<kFactored && GMPI_FWD_WIDE_FACT != 0, FwdRingWide, FwdRing>::type;
 
-template <bool kAlignCorners, bool kEmitT, bool kFactored>
-__global__ void __launch_bounds__(kStagedThreads, kCtasPerSm)
-mpi_fwd_staged_kernel(const RenderParams p, const __grid_constant__ TmaMaps maps, const int tiles_x, const int tiles_y) {
+// The staged forward, body of both kernels below.  kCut: early ray termination at T < tau (never with kEmitT); s_vote [kStages]
+// and `skipped` (nullable) as in staged_producer.  With kCut == false the extra arguments are unused and the code is that of the
+// kernel before termination existed.
+template <bool kAlignCorners, bool kEmitT, bool kFactored, bool kCut>
+__device__ __forceinline__ void fwd_staged_body(const RenderParams& p, const TmaMaps& maps, const int tiles_x, const int tiles_y,
+                                                float tau, uint32_t* s_vote, unsigned long long* skipped) {
+    static_assert(!(kCut && kEmitT), "the training forward saves every T: no termination");
     extern __shared__ __align__(1024) unsigned char smem_raw[];
     float* s_buf = reinterpret_cast<float*>(smem_raw);   // the ring starts the dynamic segment (1024-byte aligned)
     using Ring = FwdRingFor<kFactored>;
@@ -561,7 +603,9 @@ mpi_fwd_staged_kernel(const RenderParams p, const __grid_constant__ TmaMaps maps
 
     if (warp == kConsWarps) {
         NoPacer np;
-        staged_producer<kAlignCorners, Ring, kFactored>(p, maps, s_buf, s_meta, s_full, s_empty, &s_walk, lane, np);
+        if constexpr (kCut) staged_producer<kAlignCorners, Ring, kFactored, NoPacer, true>(p, maps, s_buf, s_meta, s_full, s_empty, &s_walk, lane, np,
+                                                                                          s_vote, skipped);
+        else staged_producer<kAlignCorners, Ring, kFactored>(p, maps, s_buf, s_meta, s_full, s_empty, &s_walk, lane, np);
     } else {
         // ================================ consumer warps ================================
         // warp w owns rows kPairs*w .. kPairs*w + kPairs-1 of the tile; a lane owns x = lane and lane+32 on each of them
@@ -590,7 +634,7 @@ mpi_fwd_staged_kernel(const RenderParams p, const __grid_constant__ TmaMaps maps
                 v_table = v;
             }
             if (py0 + kPairs * warp >= p.H) {      // warp-uniform: no row of this warp is inside the image
-                consumer_idle_tile(s_full, s_empty, N, lane, c_stage, c_phase);
+                consumer_idle_tile<kCut>(s_full, s_empty, N, lane, c_stage, c_phase, s_meta);
                 continue;
             }
             RayConst rc[kPix];   // scalar copies, only for the generic (rare) body and the epilogue
@@ -657,6 +701,13 @@ mpi_fwd_staged_kernel(const RenderParams p, const __grid_constant__ TmaMaps maps
                 if (!done) {
                     // ---- generic body: per-pixel range / box checks, direct sampling when not staged ----
                     const int bw = mt.sel & 0xff, mode = (mt.sel >> 8) & 3, bw4 = 4 * bw;
+                    if constexpr (kCut) {
+                        if (mode == kModeEnd) {          // the producer cut the tile short: release the stage, go to the epilogue
+                            __syncwarp();
+                            mbar_arrive_if(&s_empty[s], lane_ == 0);
+                            break;
+                        }
+                    }
                     const float fbw2 = (float)(bw - 2), fbh2 = (float)mt.rows2;
                     const float fbx0 = (float)(mt.cx - kFloorMagicBits), fby0 = (float)(mt.cy - kFloorMagicBits);
                     const float* plane = kFactored ? nullptr : p.rgba + ((size_t)m * N + i) * 4 * tex;
@@ -698,6 +749,12 @@ mpi_fwd_staged_kernel(const RenderParams p, const __grid_constant__ TmaMaps maps
                         Ts[q] -= w;
                     }
                 }
+                if constexpr (kCut) {         // the vote (see kModeEnd): one ballot, one shared OR, before the release
+                    bool alive = false;
+#pragma unroll
+                    for (int P = 0; P < kPairs; ++P) alive = alive || T[P].x >= tau || T[P].y >= tau;
+                    if (__any_sync(0xffffffffu, alive) && lane_ == 0) atomicOr(&s_vote[s], 1u);
+                }
                 __syncwarp();
                 mbar_arrive_if(&s_empty[s], lane_ == 0);    // predicated, no branch
             }
@@ -726,6 +783,22 @@ mpi_fwd_staged_kernel(const RenderParams p, const __grid_constant__ TmaMaps maps
         }
         if (flag) atomicOr(p.flags, flag);
     }
+}
+
+template <bool kAlignCorners, bool kEmitT, bool kFactored>
+__global__ void __launch_bounds__(kStagedThreads, kCtasPerSm)
+mpi_fwd_staged_kernel(const RenderParams p, const __grid_constant__ TmaMaps maps, const int tiles_x, const int tiles_y) {
+    fwd_staged_body<kAlignCorners, kEmitT, kFactored, false>(p, maps, tiles_x, tiles_y, 0.0f, nullptr, nullptr);
+}
+
+// Inference forward with early ray termination at T < tau (0 < tau < 1); skipped (nullable) accumulates the pixel-planes not
+// composited.  Same ring, same epilogues as mpi_fwd_staged_kernel<kAlignCorners, false, kFactored>.
+template <bool kAlignCorners, bool kFactored>
+__global__ void __launch_bounds__(kStagedThreads, kCtasPerSm)
+mpi_fwd_cut_kernel(const RenderParams p, const __grid_constant__ TmaMaps maps, const int tiles_x, const int tiles_y, const float tau,
+                   unsigned long long* skipped) {
+    __shared__ uint32_t s_vote[kStages];
+    fwd_staged_body<kAlignCorners, false, kFactored, true>(p, maps, tiles_x, tiles_y, tau, s_vote, skipped);
 }
 
 }  // namespace gmpi

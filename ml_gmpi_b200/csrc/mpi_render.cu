@@ -48,9 +48,11 @@ static int fail(int code, const char* fmt, ...) {
 constexpr int kFwdTileW = 32;
 constexpr int kFwdTileH = 8;
 
-template <bool kAlignCorners>
-__global__ void __launch_bounds__(kFwdTileW* kFwdTileH)
-mpi_fwd_direct_kernel(const RenderParams p) {
+// kCut: early ray termination, each pixel stops at the first plane in front of which T < p.stop_transmittance (inference only);
+// p.skipped (nullable) accumulates the planes not composited, one atomic per warp.
+template <bool kAlignCorners, bool kCut>
+__device__ __forceinline__ void fwd_direct_body(const RenderParams p) {     // (by value: by reference, ptxas schedules the
+                                                                            // kCut = false instance differently from the kernel it was)
     extern __shared__ __align__(16) unsigned char smem_raw[];
     PlaneConst* s_pc = reinterpret_cast<PlaneConst*>(smem_raw);
 
@@ -70,6 +72,7 @@ mpi_fwd_direct_kernel(const RenderParams p) {
 
     const int px = blockIdx.x * kFwdTileW + threadIdx.x;
     const int py = blockIdx.y * kFwdTileH + threadIdx.y;
+    unsigned skip = 0;      // kCut: planes this pixel did not composite
     if (px < p.W && py < p.H) {
         const size_t img = (size_t)p.H * p.W;
         const size_t pix = (size_t)py * p.W + px;
@@ -84,8 +87,17 @@ mpi_fwd_direct_kernel(const RenderParams p) {
         const bool check_last = (p.options & GMPI_CHECK_LAST_PLANE) != 0;
 
         float T = 1.0f, cr = 0.0f, cg = 0.0f, cb = 0.0f, cws = 0.0f;
+        const float tau = kCut ? p.stop_transmittance : 0.0f;
 #pragma unroll 2
         for (int i = 0; i < p.N; ++i) {
+            if (kCut && T < tau) {           // planes i.. add less than tau * max value
+                if (check_last) {            // the last-plane check still sees every pixel
+                    const TexCoord tl = plane_coord<kAlignCorners>(s_pc[p.N - 1], rc, hsx, hsy, fWt, fHt);
+                    if (!(tl.u >= -1.0f && tl.u <= 1.0f && tl.v >= -1.0f && tl.v <= 1.0f)) flag |= GMPI_FLAG_LAST_PLANE_OOB;
+                }
+                skip = (unsigned)(p.N - i);
+                break;
+            }
             const PlaneConst pc = s_pc[i];
             const PlaneChans plane = plane_chans(p, m, i, tex);
             if (p.transmittance) p.transmittance[((size_t)v * p.N + i) * img + pix] = T;   // training: T_i for the backward sweep
@@ -115,7 +127,22 @@ mpi_fwd_direct_kernel(const RenderParams p) {
         }
         store_pixel(p, v, img, pix, cr, cg, cb, dep);
     }
+    if (kCut && p.skipped) {      // one atomic per warp (a warp is one row of 32 x: all lanes reach this point)
+        const unsigned n = __reduce_add_sync(0xffffffffu, skip);
+        if (threadIdx.x == 0 && n) atomicAdd(p.skipped, (unsigned long long)n);
+    }
     if (flag) atomicOr(p.flags, flag);
+}
+
+template <bool kAlignCorners>
+__global__ void __launch_bounds__(kFwdTileW* kFwdTileH)
+mpi_fwd_direct_kernel(const RenderParams p) {
+    fwd_direct_body<kAlignCorners, false>(p);
+}
+template <bool kAlignCorners>
+__global__ void __launch_bounds__(kFwdTileW* kFwdTileH)
+mpi_fwd_direct_cut_kernel(const RenderParams p) {
+    fwd_direct_body<kAlignCorners, true>(p);
 }
 
 // ------------------------------------------------------------------------------------------
@@ -344,6 +371,16 @@ static int check_params(const RenderParams& p, bool bwd) {
         return fail(GMPI_ERR_UNSUPPORTED, "texture of %dx%d texels exceeds 2^31 elements per channel", p.Ht, p.Wt);
     if (p.view_group < 0 || (p.view_group > 1 && p.V % p.view_group != 0))
         return fail(GMPI_ERR_INVALID_ARGUMENT, "view_group=%d does not divide V=%d", p.view_group, p.V);
+    if (!(p.stop_transmittance >= 0.0f && p.stop_transmittance < 1.0f))      // (NaN fails both comparisons)
+        return fail(GMPI_ERR_INVALID_ARGUMENT, "stop_transmittance=%g must be in [0, 1)", (double)p.stop_transmittance);
+    if (p.stop_transmittance > 0.0f) {
+        if (bwd)
+            return fail(GMPI_ERR_INVALID_ARGUMENT, "stop_transmittance > 0 in the backward: gradients are exact, the backward "
+                        "composites every plane");
+        if (p.transmittance)
+            return fail(GMPI_ERR_INVALID_ARGUMENT, "stop_transmittance > 0 with a transmittance buffer: the training forward saves "
+                        "every T, termination is for inference only");
+    }
     if (bwd) {
         if (p.cam) return fail(GMPI_ERR_UNSUPPORTED, "the backward needs the reference's ray tensors (cam is forward-only)");
         if (!p.g_color) return fail(GMPI_ERR_INVALID_ARGUMENT, "null gradient pointer");
@@ -408,6 +445,15 @@ static cudaError_t launch_fwd_staged(const RenderParams& p, const TmaMaps& maps,
     kernel<<<grid, kStagedThreads, smem, st>>>(p, maps, tiles_x, tiles_y);
     return cudaSuccess;
 }
+template <bool AC, bool FAC>
+static cudaError_t launch_fwd_cut(const RenderParams& p, const TmaMaps& maps, int grid, int tiles_x, int tiles_y, cudaStream_t st) {
+    auto kernel = mpi_fwd_cut_kernel<AC, FAC>;
+    constexpr size_t smem = FwdRingFor<FAC>::kWideFact ? kStagedSmemWide : kStagedSmem;
+    cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return e;
+    kernel<<<grid, kStagedThreads, smem, st>>>(p, maps, tiles_x, tiles_y, p.stop_transmittance, p.skipped);
+    return cudaSuccess;
+}
 
 // Forward launch for a filled RenderParams.
 static int launch_fwd(RenderParams p, cudaStream_t st) {
@@ -440,7 +486,10 @@ static int launch_fwd(RenderParams p, cudaStream_t st) {
             const long n_tiles = (long)tiles_x * tiles_y * p.V;
             const int grid = (int)(n_tiles < (long)sms * kCtasPerSm ? n_tiles : (long)sms * kCtasPerSm);
             cudaError_t e;
-            if (fac) {
+            if (p.stop_transmittance > 0.0f) {      // (check_params: never together with the transmittance output)
+                if (fac) e = ac ? launch_fwd_cut<true, true>(p, maps, grid, tiles_x, tiles_y, st) : launch_fwd_cut<false, true>(p, maps, grid, tiles_x, tiles_y, st);
+                else e = ac ? launch_fwd_cut<true, false>(p, maps, grid, tiles_x, tiles_y, st) : launch_fwd_cut<false, false>(p, maps, grid, tiles_x, tiles_y, st);
+            } else if (fac) {
                 if (ac && emit) e = launch_fwd_staged<true, true, true>(p, maps, grid, tiles_x, tiles_y, st);
                 else if (ac) e = launch_fwd_staged<true, false, true>(p, maps, grid, tiles_x, tiles_y, st);
                 else if (emit) e = launch_fwd_staged<false, true, true>(p, maps, grid, tiles_x, tiles_y, st);
@@ -463,15 +512,11 @@ static int launch_fwd(RenderParams p, cudaStream_t st) {
     dim3 grid((p.W + kFwdTileW - 1) / kFwdTileW, (p.H + kFwdTileH - 1) / kFwdTileH, p.V);
     if (grid.y > 65535) return fail(GMPI_ERR_UNSUPPORTED, "image height %d too large", p.H);
     if (p.V > 65535) return fail(GMPI_ERR_UNSUPPORTED, "V=%d views exceed one launch of the direct kernel (65535); split the batch", p.V);
-    if (ac) {
-        if (smem > 48 * 1024)
-            GMPI_CUDA_OK(cudaFuncSetAttribute(mpi_fwd_direct_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        mpi_fwd_direct_kernel<true><<<grid, block, smem, st>>>(p);
-    } else {
-        if (smem > 48 * 1024)
-            GMPI_CUDA_OK(cudaFuncSetAttribute(mpi_fwd_direct_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        mpi_fwd_direct_kernel<false><<<grid, block, smem, st>>>(p);
-    }
+    const bool cut = p.stop_transmittance > 0.0f;
+    void (*kernel)(const RenderParams) = ac ? (cut ? mpi_fwd_direct_cut_kernel<true> : mpi_fwd_direct_kernel<true>)
+                                            : (cut ? mpi_fwd_direct_cut_kernel<false> : mpi_fwd_direct_kernel<false>);
+    if (smem > 48 * 1024) GMPI_CUDA_OK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    kernel<<<grid, block, smem, st>>>(p);
     GMPI_CUDA_OK(cudaGetLastError());
     return GMPI_OK;
 }
@@ -604,14 +649,22 @@ static RenderParams params_from_desc(const gmpi_render_desc* d) {
     p.M = d->M; p.V = d->V; p.N = d->N; p.Ht = d->Ht; p.Wt = d->Wt; p.H = d->H; p.W = d->W;
     p.view_group = d->view_group;
     p.options = d->options & 0xffffu;      // the upper bits are internal
+    if (d->struct_bytes >= sizeof(gmpi_render_desc)) {      // the early-termination fields (an older descriptor ends before them)
+        p.stop_transmittance = d->stop_transmittance;
+        p.skipped = reinterpret_cast<unsigned long long*>(d->skipped_pixel_planes);
+    }
     return p;
 }
 
+static constexpr size_t kDescBytesWithoutStop = offsetof(gmpi_render_desc, stop_transmittance);
+static_assert(sizeof(uint64_t) == sizeof(unsigned long long), "skip counter");
+
 static int check_desc(const gmpi_render_desc* d) {
     if (!d) return fail(GMPI_ERR_INVALID_ARGUMENT, "null descriptor");
-    if (d->struct_bytes != sizeof(gmpi_render_desc))
-        return fail(GMPI_ERR_INVALID_ARGUMENT, "gmpi_render_desc.struct_bytes = %u, this library expects %zu (ABI %d)", d->struct_bytes,
-                    sizeof(gmpi_render_desc), GMPI_ABI_VERSION);
+    // the descriptor before the early-termination fields (everything up to stop_transmittance) is accepted: they read as absent
+    if (d->struct_bytes != sizeof(gmpi_render_desc) && d->struct_bytes != kDescBytesWithoutStop)
+        return fail(GMPI_ERR_INVALID_ARGUMENT, "gmpi_render_desc.struct_bytes = %u, this library expects %zu (ABI %d) or %zu (without stop_transmittance)",
+                    d->struct_bytes, sizeof(gmpi_render_desc), GMPI_ABI_VERSION, kDescBytesWithoutStop);
     return GMPI_OK;
 }
 
@@ -969,8 +1022,9 @@ static int host_render_locked(HostCache& c, const RenderParams& h, uint32_t* fla
     float *d_dhw = (float*)(base + o_dhw), *d_ray = (float*)(base + o_ray), *d_eye = (float*)(base + o_eye), *d_z = (float*)(base + o_z);
     int32_t* d_v2m = (int32_t*)(base + o_v2m);
     uint32_t* d_flags = (uint32_t*)(base + o_flags);
+    unsigned long long* d_skipped = (unsigned long long*)(base + o_flags + 8);     // (within the 256 bytes of the flags slot)
     cudaStream_t s_copy = c.s_copy, s_run = c.s_run;
-    GMPI_CUDA_OK(cudaMemsetAsync(d_flags, 0, sizeof(uint32_t), s_run));
+    GMPI_CUDA_OK(cudaMemsetAsync(d_flags, 0, 16, s_run));
     GMPI_CUDA_OK(cudaMemsetAsync(d_v2m, 0, sizeof(int32_t) * (size_t)(V > 0 ? V : 1), s_run));   // a staged MPI is slot-local index 0
     GMPI_CUDA_OK(cudaMemcpyAsync(d_dhw, h.dhw, sizeof(float) * (size_t)M * N * 3, cudaMemcpyHostToDevice, s_run));
     if (h.cam) {
@@ -1014,6 +1068,7 @@ static int host_render_locked(HostCache& c, const RenderParams& h, uint32_t* fla
             p.depth = (float*)(base + o_depth) + (size_t)v0 * img;
         }
         p.flags = d_flags;
+        p.skipped = h.skipped ? d_skipped : nullptr;
         p.view_group = (M == 1 && h.view_group > 1) ? h.view_group : 1;
         rc = launch_fwd(p, s_run);
         if (rc) return rc;
@@ -1030,8 +1085,11 @@ static int host_render_locked(HostCache& c, const RenderParams& h, uint32_t* fla
         GMPI_CUDA_OK(cudaMemcpyAsync(h.depth, base + o_depth, sizeof(float) * (size_t)V * img, cudaMemcpyDeviceToHost, s_run));
     }
     GMPI_CUDA_OK(cudaMemcpyAsync(flags_out, d_flags, sizeof(uint32_t), cudaMemcpyDeviceToHost, s_run));
+    unsigned long long skipped = 0;
+    if (h.skipped) GMPI_CUDA_OK(cudaMemcpyAsync(&skipped, d_skipped, sizeof(skipped), cudaMemcpyDeviceToHost, s_run));
     GMPI_CUDA_OK(cudaStreamSynchronize(s_run));
     GMPI_CUDA_OK(cudaStreamSynchronize(s_copy));
+    if (h.skipped) *h.skipped += skipped;      // accumulated into, like the device counter
     return GMPI_OK;
 }
 

@@ -36,7 +36,7 @@ class _RenderFn(torch.autograd.Function):
     The MPI is either expanded (`rgba`) or factored (`rgb`, `alpha`, optional `bg_rgb`); the unused form is None."""
 
     @staticmethod
-    def forward(ctx, rgba, rgb, alpha, bg_rgb, dhw, view2mpi, ray_dir, eye, z_dir, options, flags, view_group):
+    def forward(ctx, rgba, rgb, alpha, bg_rgb, dhw, view2mpi, ray_dir, eye, z_dir, options, flags, view_group, stop_transmittance):
         lib = _lib.load()
         factored = rgba is None
         ref = alpha if factored else rgba
@@ -51,10 +51,14 @@ class _RenderFn(torch.autograd.Function):
         trans = None
         if any(ctx.needs_input_grad[:4]):
             trans = torch.empty((V, N, H, W), device=dev, dtype=torch.float32)
+        # early ray termination only when no input needs a gradient: with one the render is exact (the backward needs every
+        # plane's T), so one MPI object serves the no-grad D step and the G step alike
+        tau = float(stop_transmittance) if trans is None else 0.0
         with torch.cuda.device(dev):
             d = _lib.make_desc(options=options, M=M, V=V, N=N, Ht=Ht, Wt=Wt, H=H, W=W, view_group=view_group, rgba=rgba, rgb=rgb,
                                alpha=alpha, bg_rgb=bg_rgb, view2mpi=view2mpi, dhw=dhw, ray_dir=ray_dir, eye=eye, z_dir=z_dir,
-                               color=color, depth=depth, transmittance=trans, flags=flags, stream=_stream_ptr(dev))
+                               color=color, depth=depth, transmittance=trans, flags=flags, stream=_stream_ptr(dev),
+                               stop_transmittance=tau)
             _lib.check(lib.gmpi_mpi_render_fwd_ex(ctypes.byref(d)))
         ctx.save_for_backward(rgba, rgb, alpha, bg_rgb, dhw, view2mpi, ray_dir, eye, z_dir, trans)
         ctx.options, ctx.view_group = options, view_group
@@ -65,7 +69,7 @@ class _RenderFn(torch.autograd.Function):
     @torch.autograd.function.once_differentiable     # raw kernels: a double backward (create_graph=True) must raise, not
     def backward(ctx, g_color, g_depth):             # silently treat the result as constant (the reference's R1 only differentiates D)
         rgba, rgb, alpha, bg_rgb, dhw, view2mpi, ray_dir, eye, z_dir, trans = ctx.saved_tensors
-        none = (None,) * 12
+        none = (None,) * 13
         if not any(ctx.needs_input_grad[:4]):
             return none
         lib = _lib.load()
@@ -94,7 +98,7 @@ class _RenderFn(torch.autograd.Function):
                                ray_dir=ray_dir, eye=eye, z_dir=z_dir, transmittance=trans, g_color=g_color, g_depth=g_depth,
                                g_rgba=g_rgba, g_rgb=g_rgb, g_bg_rgb=g_bg, g_alpha=g_alpha, stream=_stream_ptr(dev))
             _lib.check(lib.gmpi_mpi_render_bwd_ex(ctypes.byref(d)))
-        return (g_rgba, g_rgb, g_alpha, g_bg) + (None,) * 8
+        return (g_rgba, g_rgb, g_alpha, g_bg) + (None,) * 9
 
 
 _warned_direct = set()
@@ -120,28 +124,40 @@ def _options(align_corners, check_last_plane, color_minus1_1, u8_round=False):
         | (_lib.OPT_COLOR_MINUS1_1 if color_minus1_1 else 0) | (_lib.OPT_U8_ROUND_HALF_UP if u8_round else 0)
 
 
+def _check_stop(stop_transmittance) -> float:
+    tau = float(stop_transmittance)
+    if not 0.0 <= tau < 1.0:
+        raise ValueError(f"stop_transmittance must be in [0, 1), got {stop_transmittance}")
+    return tau
+
+
 def render_views(rgba, dhw, view2mpi, ray_dir, eye, z_dir, *, align_corners=True, check_last_plane=False,
-                 color_minus1_1=False, flags: Optional[torch.Tensor] = None, view_group: int = 1):
+                 color_minus1_1=False, flags: Optional[torch.Tensor] = None, view_group: int = 1, stop_transmittance: float = 0.0):
     """Functional form on packed tensors (no list handling, no host sync).
     rgba [M,N,4,Ht,Wt], dhw [M,N,3], view2mpi [V] int32, ray_dir [V,3,H,W], eye/z_dir [V,3].
     Returns (color [V,3,H,W], depth [V,1,H,W]); `flags` (uint32 tensor of 1, int32 storage) is OR-ed into.
-    view_group > 1: every view_group consecutive views share one MPI (tile-order hint: L2 reuse, see the C header)."""
+    view_group > 1: every view_group consecutive views share one MPI (tile-order hint: L2 reuse, see the C header).
+    stop_transmittance = tau in (0, 1): early ray termination when no input needs a gradient -- a pixel may drop the planes
+    behind the point where its transmittance fell below tau, so every output is within tau * max(value) below the exact one
+    (the contract in include/gmpi_mpi_render.h).  0 (default): exact.  Ignored (exact render) when rgba requires grad."""
     if not rgba.is_cuda:
         raise RuntimeError("ml_gmpi_b200 renders on CUDA devices only (no CPU fallback); got a CPU tensor")
     if flags is None:
         flags = torch.zeros(1, dtype=torch.int32, device=rgba.device)
     _warn_if_direct(rgba, ray_dir.shape[0], ray_dir.shape[2], ray_dir.shape[3])
     return _RenderFn.apply(_as_f32c(rgba), None, None, None, _as_f32c(dhw), view2mpi, _as_f32c(ray_dir), _as_f32c(eye), _as_f32c(z_dir),
-                           _options(align_corners, check_last_plane, color_minus1_1), flags, int(view_group))
+                           _options(align_corners, check_last_plane, color_minus1_1), flags, int(view_group),
+                           _check_stop(stop_transmittance))
 
 
 def render_views_factored(rgb, alpha, dhw, view2mpi, ray_dir, eye, z_dir, *, bg_rgb=None, align_corners=True,
-                          check_last_plane=False, color_minus1_1=False, flags: Optional[torch.Tensor] = None, view_group: int = 1):
+                          check_last_plane=False, color_minus1_1=False, flags: Optional[torch.Tensor] = None, view_group: int = 1,
+                          stop_transmittance: float = 0.0):
     """The same render from the generator's FACTORED output (networks_cond_on_pos_enc.py:950-975,984): one colour image
     rgb [M,3,Ht,Wt] shared by all planes (bg_rgb [M,3,Ht,Wt]: the last plane's own colour under torgba_sep_background) and
     alpha [M,N,1,Ht,Wt] -- what the reference expands to [M,N,4,Ht,Wt] (and copies per view, train.py:553-558,733-738) before
     rendering.  Output identical to render_views on the expanded stack, 4x fewer HBM bytes; differentiable w.r.t. rgb, alpha
-    and bg_rgb (d/d rgb is the sum over the planes that share it)."""
+    and bg_rgb (d/d rgb is the sum over the planes that share it).  stop_transmittance: as in render_views."""
     if not alpha.is_cuda:
         raise RuntimeError("ml_gmpi_b200 renders on CUDA devices only (no CPU fallback); got a CPU tensor")
     assert rgb.ndim == 4 and rgb.shape[1] == 3 and alpha.ndim == 5 and alpha.shape[2] == 1 and rgb.shape[0] == alpha.shape[0] \
@@ -152,7 +168,7 @@ def render_views_factored(rgb, alpha, dhw, view2mpi, ray_dir, eye, z_dir, *, bg_
     _warn_if_direct(alpha, ray_dir.shape[0], ray_dir.shape[2], ray_dir.shape[3])
     return _RenderFn.apply(None, _as_f32c(rgb), _as_f32c(alpha), None if bg_rgb is None else _as_f32c(bg_rgb), _as_f32c(dhw), view2mpi,
                            _as_f32c(ray_dir), _as_f32c(eye), _as_f32c(z_dir), _options(align_corners, check_last_plane, color_minus1_1),
-                           flags, int(view_group))
+                           flags, int(view_group), _check_stop(stop_transmittance))
 
 
 def expand_factored(rgb, alpha, bg_rgb=None):
@@ -167,11 +183,14 @@ def expand_factored(rgb, alpha, bg_rgb=None):
 
 def render_frames(*, dhw, view2mpi, rgba=None, rgb=None, alpha=None, bg_rgb=None, ray_dir=None, eye=None, z_dir=None, cam=None,
                   align_corners=True, check_last_plane=False, video: Optional[dict] = None, u8_round=False,
-                  flags: Optional[torch.Tensor] = None, view_group: int = 1, H: Optional[int] = None, W: Optional[int] = None):
+                  flags: Optional[torch.Tensor] = None, view_group: int = 1, H: Optional[int] = None, W: Optional[int] = None,
+                  stop_transmittance: float = 0.0, skipped: Optional[torch.Tensor] = None):
     """Inference-only render with the opt-in fast paths of the C ABI (no autograd):
       cam [V,16]     rays generated in the kernel from the pinhole camera (see camera.cam_params) instead of ray_dir/eye/z_dir;
       video={"near": ray_start, "far": ray_end, "depth": True}   uint8 HWC frames as render_video.py:118-126 builds them:
                      returns (rgb_u8 [V,H,W,3], depth_u8 [V,H,W,1] or None); otherwise (color in [-1,1], depth) fp32.
+      stop_transmittance = tau in (0, 1)   early ray termination (see render_views; the [-1,1] colour moves by up to 2 tau);
+      skipped        int64 CUDA tensor of one element: the number of pixel-planes not composited is added to it.
     """
     ref = alpha if rgba is None else rgba
     if not ref.is_cuda:
@@ -189,6 +208,9 @@ def render_frames(*, dhw, view2mpi, rgba=None, rgb=None, alpha=None, bg_rgb=None
         ray_dir, eye, z_dir = _as_f32c(ray_dir), _as_f32c(eye), _as_f32c(z_dir)
     if flags is None:
         flags = torch.zeros(1, dtype=torch.int32, device=dev)
+    tau = _check_stop(stop_transmittance)
+    if skipped is not None and not (skipped.is_cuda and skipped.dtype == torch.int64 and skipped.numel() == 1 and skipped.is_contiguous()):
+        raise ValueError("skipped must be a contiguous int64 CUDA tensor of one element")
     color = depth = v_rgb = v_depth = None
     near = rng = 0.0
     if video is not None:
@@ -205,7 +227,8 @@ def render_frames(*, dhw, view2mpi, rgba=None, rgb=None, alpha=None, bg_rgb=None
         d = _lib.make_desc(options=_options(align_corners, check_last_plane, True, u8_round), M=M, V=V, N=N, Ht=Ht, Wt=Wt, H=H, W=W,
                            view_group=int(view_group), depth_near=near, depth_range=rng, rgba=keep[0], rgb=keep[1], alpha=keep[2],
                            bg_rgb=keep[3], view2mpi=view2mpi, dhw=keep[4], ray_dir=ray_dir, eye=eye, z_dir=z_dir, cam=cam, color=color,
-                           depth=depth, video_rgb=v_rgb, video_depth=v_depth, flags=flags, stream=_stream_ptr(dev))
+                           depth=depth, video_rgb=v_rgb, video_depth=v_depth, flags=flags, stream=_stream_ptr(dev),
+                           stop_transmittance=tau, skipped_pixel_planes=skipped)
         _lib.check(lib.gmpi_mpi_render_fwd_ex(ctypes.byref(d)))
     return (v_rgb, v_depth) if video is not None else (color, depth)
 
@@ -226,13 +249,16 @@ class MPI(nn.Module):
          "defer" the geometric flags are still computed inside the render kernel (free) but nothing
                  is scanned or synced; read them later with `.raise_if_flagged()`;
          "off"   like "defer" without the last-plane check.
+    `stop_transmittance` = tau in (0, 1): early ray termination of renders where no input needs a gradient (see render_views);
+    renders with a gradient stay exact.  0 (default): exact.
     """
 
-    def __init__(self, align_corners=True, validate: str = "full"):
+    def __init__(self, align_corners=True, validate: str = "full", stop_transmittance: float = 0.0):
         super().__init__()
         assert validate in ("full", "defer", "off"), validate
         self._align_corners = align_corners
         self.validate = validate
+        self.stop_transmittance = _check_stop(stop_transmittance)
         self._flags = None
         self._flag_ctx = None
 
@@ -297,7 +323,8 @@ class MPI(nn.Module):
         color, depth = render_views(rgba, batch_dhw.to(dev), view2mpi, ray_dir.to(dev), eye.to(dev), z_dir.to(dev),
                                     align_corners=self._align_corners,
                                     check_last_plane=bool(assert_not_out_of_last_plane) and self.validate != "off",
-                                    flags=flags, view_group=self.view_group_of(batch_ray_dir))
+                                    flags=flags, view_group=self.view_group_of(batch_ray_dir),
+                                    stop_transmittance=self.stop_transmittance)
         self._flags = flags
         self._flag_ctx = (batch_dhw, eye, c2w_mat, sphere_c)
         if self.validate == "full":

@@ -35,7 +35,7 @@ def sweep_angles(n_views: int = 100, horizontal: bool = True, mean: float = 0.0)
     return [float(a) + mean for a in np.linspace(half, -half, n_views).tolist()]
 
 
-def _default_video_render(rgba, dhw, c2w, img_size, fov_deg, near, far, fast_rays, factored):
+def _default_video_render(rgba, dhw, c2w, img_size, fov_deg, near, far, fast_rays, factored, stop_transmittance=0.0):
     from .mpi import render_frames
     dev = dhw.device
     V = c2w.shape[0]
@@ -44,20 +44,23 @@ def _default_video_render(rgba, dhw, c2w, img_size, fov_deg, near, far, fast_ray
     if fast_rays:
         cam = cam_params(c2w.to(dev), focal_from_fov(fov_deg, img_size), img_size, img_size)
         return render_frames(dhw=dhw, view2mpi=v2m, cam=cam, H=img_size, W=img_size, video={"near": near, "far": far},
-                             check_last_plane=True, view_group=V, **kw)
+                             check_last_plane=True, view_group=V, stop_transmittance=stop_transmittance, **kw)
     ray_dir, eye, z_dir = PinholeCamera.from_fov(fov_deg, img_size, img_size).generate_rays(c2w.to(dev))
     return render_frames(dhw=dhw, view2mpi=v2m, ray_dir=ray_dir, eye=eye, z_dir=z_dir, video={"near": near, "far": far},
-                         check_last_plane=True, view_group=V, **kw)
+                         check_last_plane=True, view_group=V, stop_transmittance=stop_transmittance, **kw)
 
 
 def render_video_frames(mpi_rgba: Optional[torch.Tensor], dhw: torch.Tensor, angles: Sequence[float], *, img_size: int, fov_deg: float,
                         ray_start: float, ray_end: float, sphere_center, sphere_r: float, horizontal: bool = True,
                         other_angle: float = 0.0, fast_rays: bool = False, factored: Optional[Tuple] = None,
-                        rank: int = 0, world: int = 1, gather: bool = True, render_fn: Optional[Callable] = None):
+                        rank: int = 0, world: int = 1, gather: bool = True, render_fn: Optional[Callable] = None,
+                        stop_transmittance: float = 0.0):
     """All `angles` (yaw sweep if `horizontal`, else pitch sweep; the other angle fixed) of ONE MPI ([1,N,4,T,T], or
     factored=(rgb [1,3,T,T], alpha [1,N,1,T,T], bg_rgb or None)) as uint8 frames.
     Returns (img [V,H,W,3] uint8, depth [V,H,W,1] uint8) as CPU tensors: all V views when `gather` (every rank), else this rank's
-    slice [lo, hi) of shard_range(V, rank, world)."""
+    slice [lo, hi) of shard_range(V, rank, world).
+    stop_transmittance: early ray termination of the render (see mpi.render_views); handed to `render_fn` as a keyword
+    argument when it is not 0, so render functions without the parameter keep working for exact renders."""
     V = len(angles)
     lo, hi = shard_range(V, rank, world)
     a = torch.tensor(list(angles[lo:hi]), dtype=torch.float32).reshape(-1, 1)
@@ -66,7 +69,8 @@ def render_video_frames(mpi_rgba: Optional[torch.Tensor], dhw: torch.Tensor, ang
     c2w = sphere_poses(yaws, pitches, sphere_center, sphere_r)
     fn = render_fn or _default_video_render
     if hi > lo:
-        img, depth = fn(mpi_rgba, dhw, c2w, img_size, fov_deg, ray_start, ray_end, fast_rays, factored)
+        extra = {"stop_transmittance": float(stop_transmittance)} if stop_transmittance else {}
+        img, depth = fn(mpi_rgba, dhw, c2w, img_size, fov_deg, ray_start, ray_end, fast_rays, factored, **extra)
     else:
         dev = dhw.device
         img = torch.empty((0, img_size, img_size, 3), dtype=torch.uint8, device=dev)

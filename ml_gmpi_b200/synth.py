@@ -60,3 +60,36 @@ def make_case(*, n_planes, tex, img, n_mpi, views_per_mpi=1, seed=1234, device="
     dhw = ffhq_dhw(n_planes).to(device).unsqueeze(0).expand(n_mpi, -1, -1).contiguous()
     v2m = torch.arange(n_mpi, dtype=torch.int32, device=device).repeat_interleave(views_per_mpi)
     return Case(t, dhw, v2m, ray_dir, eye, z_dir, c2w, yaws, pitches)
+
+
+def surface_alpha(n_mpi, n_planes, tex, *, device="cpu", front=0.2, back=0.75, band=6.0, peak=0.98, semi_axes=(0.55, 0.7)):
+    """Alpha [M,N,1,T,T] of a "head": an ellipsoid heightfield over the texture centre, nearest (plane front*N) at the centre and
+    reaching plane back*N at its rim; in front of the surface alpha = 0, then a soft band (alpha rising to `peak` over the first
+    quarter of `band` planes, zero after it); outside the ellipse alpha = 0; the last plane alpha = 1 everywhere.  A stand-in for
+    a trained generator's MPI: only rays through the head become opaque before the last plane."""
+    u = torch.linspace(-1.0, 1.0, tex, device=device)
+    r2 = (u.view(1, -1) / semi_axes[0]) ** 2 + (u.view(-1, 1) / semi_axes[1]) ** 2          # [T(y), T(x)]
+    inside = r2 < 1.0
+    s = (back - (back - front) * torch.sqrt(torch.clamp(1.0 - r2, min=0.0))) * (n_planes - 1)  # surface plane index
+    i = torch.arange(n_planes, device=device, dtype=torch.float32).view(-1, 1, 1)
+    d = i - s.unsqueeze(0)                                                                     # planes behind the surface
+    a = torch.clamp((d + 1.0) / (0.25 * band), 0.0, 1.0) * peak * (d < band).float() * inside.unsqueeze(0).float()
+    a[-1] = 1.0
+    return a.unsqueeze(0).unsqueeze(2).expand(n_mpi, -1, -1, -1, -1).contiguous()
+
+
+def make_workload(kind, *, n_planes, tex, img, n_mpi, views_per_mpi=1, seed=1234, device="cpu", yaws=None, pitches=None) -> Case:
+    """Early-ray-termination workloads, random colours and last plane alpha = 1 in all three:
+      "noise"   white-noise alpha (make_case(last_alpha_one=True)): T falls below 2^-24 after a few dozen planes everywhere;
+      "surface" surface_alpha: only tiles inside the head can terminate;
+      "empty"   alpha = 0 except the last plane: nothing can be skipped (the cost of the termination test alone)."""
+    case = make_case(n_planes=n_planes, tex=tex, img=img, n_mpi=n_mpi, views_per_mpi=views_per_mpi, seed=seed, device=device,
+                     last_alpha_one=True, yaws=yaws, pitches=pitches)
+    if kind == "surface":
+        case.rgba[:, :, 3:] = surface_alpha(n_mpi, n_planes, tex, device=device)
+    elif kind == "empty":
+        case.rgba[:, :, 3] = 0.0
+        case.rgba[:, -1, 3] = 1.0
+    elif kind != "noise":
+        raise ValueError(f"unknown workload {kind!r}")
+    return case

@@ -237,6 +237,40 @@ int gmpi_mpi_render_bwd_ex(const gmpi_render_desc* desc);
 int gmpi_mpi_render_host_ex(const gmpi_render_desc* desc, int device);
 
 /*
+ * Empty-space skipping of the INFERENCE forward: planes whose alpha is (near) zero under a whole 64x30 tile are not fetched and
+ * not composited.  Two steps on the same stream:
+ *
+ * gmpi_mpi_occupancy: one bit per 8x8-texel block of every alpha plane, set iff some alpha of the block has !(|alpha| <=
+ *   threshold) (so NaN counts as occupied, -0.0 does not).  occupancy [M][N][ceil(Ht/8)][ceil(Wt/512)] uint64 (device memory):
+ *   bit b of word w of block row r covers texels x in [8(64w+b), 8(64w+b)+8), y in [8r, 8r+8); texels outside the texture do not
+ *   exist and never set a bit.  gmpi_mpi_occupancy_plane_words(Ht, Wt) = ceil(Ht/8) * ceil(Wt/512), the words of one plane (0 for
+ *   sizes < 1).  Alpha of plane i of MPI m is read at alpha[m * mpi_stride + i * plane_stride + texel] as in gmpi_mpi_alpha_depth_fwd:
+ *   the expanded stack (alpha = rgba + 3*Ht*Wt, plane_stride = 4*Ht*Wt, mpi_stride = N*4*Ht*Wt) or the factored alpha [M,N,1,Ht,Wt]
+ *   (plane_stride = Ht*Wt).  Every word is written (no zeroing needed).  A streaming read of the alpha planes only.  Rejected
+ *   (GMPI_ERR_INVALID_ARGUMENT, before any CUDA call): threshold NaN, < 0 or >= 1.
+ *
+ * gmpi_mpi_render_fwd_skip_ex: gmpi_mpi_render_fwd_ex on the same descriptor (every option composes: expanded or factored MPI,
+ *   ray_dir or cam, fp32 / 2c-1 / uint8 video outputs, fused gather, view_group, stop_transmittance), except that the staged
+ *   kernel may skip a (tile, plane) whose staged box (the footprint estimate of the tile, rounded up to the box the kernel would
+ *   fetch) has no bit set in `occupancy`, built for the same MPI tensors.  A warp whose taps all lie in such a box composites
+ *   nothing for that plane; any other pixel samples the plane as usual, so results never depend on the footprint estimate.
+ *   The direct kernel ignores the map (exact render, nothing counted).
+ *   empty_pixel_planes: nullable uint64 [1], device memory: accumulated into (not zeroed), the in-image pixels of each tile times
+ *   the planes published empty for it.  Deterministic.
+ *   Contract.  For finite inputs, threshold 0 gives output bit-identical to gmpi_mpi_render_fwd_ex with the same descriptor,
+ *   including with stop_transmittance > 0: a plane whose taps all have alpha = 0 adds fma(0, x, acc) = acc and leaves T unchanged,
+ *   so the termination votes, decisions and count are identical too.  With threshold eps > 0, for MPIs with alpha and colour in
+ *   [0, 1] (the range the reference asserts), every output moves by at most N * eps * max(value) plus fp32 rounding (twice that
+ *   for 2c-1 colour): skipping plane j changes the composite by T_j * alpha_j * (c_j - C_behind).
+ *   Rejected (GMPI_ERR_INVALID_ARGUMENT, before any CUDA call): a NULL occupancy; a non-NULL transmittance (the training forward
+ *   stays exact).
+ */
+size_t gmpi_mpi_occupancy_plane_words(int Ht, int Wt);
+int gmpi_mpi_occupancy(const float* alpha, long long mpi_stride, long long plane_stride, int M, int N, int Ht, int Wt, float threshold,
+                       uint64_t* occupancy, void* stream);
+int gmpi_mpi_render_fwd_skip_ex(const gmpi_render_desc* desc, const uint64_t* occupancy, uint64_t* empty_pixel_planes);
+
+/*
  * LightRenderer (gmpi/core/light_renderer.py), the lighting augmentation applied to the MPI right before the render call in
  * training (train.py:534-541,702-709).  Two streaming kernels replace what the reference materialises:
  *

@@ -29,6 +29,7 @@ EXPORTS = [
     "gmpi_mpi_render_fwd_plan", "gmpi_mpi_render_fwd_ex", "gmpi_mpi_render_bwd_ex", "gmpi_mpi_render_host_ex",
     "gmpi_debug_tile_walk_ex", "gmpi_debug_cam_rays",
     "gmpi_mpi_zero_async", "gmpi_mpi_alpha_depth_fwd", "gmpi_mpi_alpha_depth_bwd", "gmpi_mpi_apply_shading_fwd", "gmpi_mpi_apply_shading_bwd",
+    "gmpi_mpi_occupancy_plane_words", "gmpi_mpi_occupancy", "gmpi_mpi_render_fwd_skip_ex",
 ]
 
 OPT_U8_ROUND_HALF_UP = 16
@@ -140,6 +141,12 @@ def load():
     lib.gmpi_mpi_apply_shading_bwd.argtypes = [vp, vp, vp, vp, vp, i, i, i, i, vp]
     lib.gmpi_mpi_render_host_ex.restype = i
     lib.gmpi_mpi_render_host_ex.argtypes = [ctypes.POINTER(RenderDesc), i]
+    lib.gmpi_mpi_occupancy_plane_words.restype = ctypes.c_size_t
+    lib.gmpi_mpi_occupancy_plane_words.argtypes = [i, i]
+    lib.gmpi_mpi_occupancy.restype = i
+    lib.gmpi_mpi_occupancy.argtypes = [vp, ll, ll, i, i, i, i, ctypes.c_float, vp, vp]
+    lib.gmpi_mpi_render_fwd_skip_ex.restype = i
+    lib.gmpi_mpi_render_fwd_skip_ex.argtypes = [ctypes.POINTER(RenderDesc), vp, vp]
     if lib.gmpi_abi_version() != ABI_VERSION:
         raise GmpiLibraryError(f"ABI mismatch: library {lib.gmpi_abi_version()} != binding {ABI_VERSION}; rebuild")
     _lib = lib

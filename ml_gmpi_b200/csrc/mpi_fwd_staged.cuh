@@ -68,7 +68,8 @@ struct __align__(16) StageMeta {
                            // down) - cx is floor(x) relative to the box
     int rows2;             // staged rows - 2: a footprint with north-west tap (rx, ry) fits iff 0<=rx<=bw-2, 0<=ry<=rows-2
     int sel;               // bits 0-7 staged width (row pitch = 4*bw floats), bits 8-9 mode (0 staged, 1 nothing under the
-                           // tile, 2 sample from global, 3 end of tile: early ray termination, see kModeEnd), bits 16-20 width
+                           // tile, 2 sample from global, 3 end of tile: early ray termination, see kModeEnd; the kSkip forward
+                           // reads bits 8-10, 4 = empty box, see kModeEmpty), bits 16-20 width
                            // class for the packed fast body, ONE-HOT (a chain of single-bit tests, most frequent first, is
                            // shorter than a jump table), or 0 (not usable: mode != 0, or plane constants outside the
                            // exact-division range)
@@ -80,6 +81,14 @@ struct __align__(16) StageMeta {
 // planes in flight, see it in the generic body, release the stage and go to the epilogue.  The producer alone decides, so the
 // ring stays in lockstep and the result does not depend on timing.
 constexpr int kModeEnd = 3;
+// Empty-space skipping (the kSkip forward, inference only): the producer tests the occupancy bits (one per 8x8 texels, see
+// gmpi_mpi_occupancy) of exactly the box it would stage, width class x staged rows clipped to the texture.  If none is set, every
+// alpha in the box is within the threshold of 0, and it publishes the box's header with this mode instead: no copies, no tx
+// bytes.  A consumer warp whose taps all lie in that box composites nothing for the plane (a = 0 leaves colour, depth and T
+// unchanged, bit for bit); a warp with a tap outside it, or with rays outside the fast range, takes the generic body and samples
+// the plane from global memory.  Only mode-0 boxes of planes whose constants allow the packed fast body become empty.  The mode
+// field is 3 bits wide in this kernel only.
+constexpr int kModeEmpty = 4;
 
 // ---- packed dual-fp32 arithmetic (sm_100 FFMA2/FADD2/FMUL2): one issue slot for two pixels, IEEE rn per element ----
 typedef float2 f2;
@@ -225,6 +234,22 @@ __device__ __forceinline__ bool sample_pairs(const float* __restrict__ sb, int c
     return true;
 }
 
+// The box test of sample_pairs alone, with a run-time width (an empty box, kModeEmpty, has no taps to take): true iff the four
+// bilinear footprints of every pixel of the warp lie inside the box of width bw2 + 2 and rows2 + 2 rows at (cx, cy).
+__device__ __forceinline__ bool taps_in_box(const CoordPairs& c, int cx, int cy, int bw2, int rows2) {
+    const f2 magic = splat(kFloorMagic);
+    bool inbox = true;
+#pragma unroll
+    for (int P = 0; P < kPairs; ++P) {
+        const f2 tx = add2_rm(c.ix[P], magic), ty = add2_rm(c.iy[P], magic);
+        const int rxa = __float_as_int(tx.x) - cx, rxb = __float_as_int(tx.y) - cx;
+        const int rya = __float_as_int(ty.x) - cy, ryb = __float_as_int(ty.y) - cy;
+        inbox = inbox && (unsigned)rxa <= (unsigned)bw2 && (unsigned)rxb <= (unsigned)bw2 && (unsigned)rya <= (unsigned)rows2 &&
+                (unsigned)ryb <= (unsigned)rows2;
+    }
+    return __all_sync(0xffffffffu, inbox);
+}
+
 // Rare path (a ray whose footprint is not in the staged box): sample the plane from global memory.  Out of line so
 // that it does not cost registers in the hot loop.
 // Expanded MPI: ONE base pointer crosses the call.  (Passing the four channel pointers of PlaneChans instead -- 8 registers that
@@ -304,8 +329,8 @@ struct TileWalk {
 };
 
 // A consumer warp without a single row inside the image: hand every stage of this tile straight back to the producer (kCut: up to
-// and including an end-of-tile header; such a warp does not vote).
-template <bool kCut = false>
+// and including an end-of-tile header; such a warp does not vote).  kModeMask: the width of the header's mode field.
+template <bool kCut = false, int kModeMask = 3>
 __device__ __forceinline__ void consumer_idle_tile(uint64_t* s_full, uint64_t* s_empty, int N, int lane, int& c_stage, uint32_t& c_phase,
                                                    const StageMeta* s_meta = nullptr) {
     for (int i = 0; i < N; ++i) {
@@ -314,7 +339,7 @@ __device__ __forceinline__ void consumer_idle_tile(uint64_t* s_full, uint64_t* s
         if (++c_stage == kStages) { c_stage = 0; c_phase ^= 1u; }
         mbar_wait(&s_full[s], ph);
         bool end = false;
-        if constexpr (kCut) end = ((s_meta[s].sel >> 8) & 3) == kModeEnd;
+        if constexpr (kCut) end = ((s_meta[s].sel >> 8) & kModeMask) == kModeEnd;
         __syncwarp();
         mbar_arrive_if(&s_empty[s], lane == 0);
         if (end) break;
@@ -373,10 +398,17 @@ struct NoPacer { static constexpr bool kActive = false; };      // the forward's
 // to do); at_end() after the last tile.
 // kCut (forward only): early ray termination, see kModeEnd.  s_vote[kStages] are the stages' vote words; `skipped` (nullable)
 // accumulates the pixel-planes of the tiles it cuts short.
-template <bool kAlignCorners, class Ring, bool kFact, class Pacer, bool kCut = false>
+// kSkip (forward only): empty-space skipping, see kModeEmpty.  occ is the occupancy map of the MPI ([M][N][ceil(Ht/8)][ceil(Wt/512)]
+// words); `skipped_empty` (nullable) accumulates the in-image pixels of a tile times the planes published empty.
+template <bool kAlignCorners, class Ring, bool kFact, class Pacer, bool kCut = false, bool kSkip = false>
 __device__ __forceinline__ void staged_producer(const RenderParams& p, const TmaMaps& maps, float* s_buf, StageMeta* s_meta,
                                             uint64_t* s_full, uint64_t* s_empty, const TileWalk* s_walk, int lane, Pacer& pacer,
-                                            uint32_t* s_vote = nullptr, unsigned long long* skipped = nullptr) {
+                                            uint32_t* s_vote = nullptr, unsigned long long* skipped = nullptr,
+                                            const uint64_t* __restrict__ occ = nullptr, unsigned long long* skipped_empty = nullptr) {
+    static_assert(!(kSkip && Ring::kReverse), "empty-space skipping is a forward-only mode");
+    // the words a box can touch: lane = 2 * (block row - first) + (word - first); a box spans at most 2 words of 64 blocks
+    static_assert((Ring::kBoxMaxH + 7) / 8 + 1 <= 16 && kWideBW / 8 + 1 <= 64, "a staged box spans <= 16 block rows x 2 words");
+    const int occ_wy = (p.Ht + 7) >> 3, occ_wx = (p.Wt + 511) >> 9;      // words per plane: block rows x words per row
     constexpr bool kReverse = Ring::kReverse;
     constexpr int kStride = Ring::kStride;      // floats per ring stage
     constexpr int kTileH = Ring::kTileRows, kStages = Ring::kRingStages, kMaxBH = Ring::kBoxMaxH, kStageFloats = Ring::kPlaneFloats;
@@ -404,6 +436,7 @@ __device__ __forceinline__ void staged_producer(const RenderParams& p, const Tma
         float crx, cry, crz;
         load_ray(p, v, cx, cy, img, crx, cry, crz);
         const RayConst rc = make_ray_const(crx, cry, crz, ev, zd);
+        unsigned n_empty = 0;       // kSkip: planes of this tile published empty
         for (int ii = 0; ii < N; ++ii) {
             const int i = kReverse ? N - 1 - ii : ii;
             const int s = p_stage;
@@ -429,8 +462,28 @@ __device__ __forceinline__ void staged_producer(const RenderParams& p, const Tma
             // width class k (tensor-map slot, one-hot bit 16 + k of the header); wide rings: slot 1 = 64, slot 4 = kWideBW
             const int k = mode != 0 ? 0 : kWide ? (need_w <= 64 ? 1 : 4) : max(0, (need_w - kMinBW + kBWStep - 1) / kBWStep);
             const int bw = (kWide && k == 4) ? kWideBW : kMinBW + k * kBWStep;
-            const int n_ops = mode == 0 ? (need_h + kRowsPerOp - 1) / kRowsPerOp : 0;
+            int n_ops = mode == 0 ? (need_h + kRowsPerOp - 1) / kRowsPerOp : 0;
             const int rows = n_ops * kRowsPerOp;
+            uint64_t occ_w = 0;     // kSkip: this lane's occupancy word of the box, masked to the box's blocks
+            if constexpr (kSkip) {
+                // Issued before the wait for a free stage, consumed after it: the load is off the ring's critical path.
+                const int x0 = max(bx0, 0), x1 = min(bx0 + bw, Wt) - 1;      // the published box, clipped to the texture
+                const int y0 = max(by0, 0), y1 = min(by0 + rows, Ht) - 1;
+                const int br = (y0 >> 3) + (lane >> 1), bxl = x0 >> 3, bxh = x1 >> 3, wx = (bxl >> 6) + (lane & 1);
+                if (mode == 0 && x0 <= x1 && y0 <= y1 && br <= (y1 >> 3) && wx <= (bxh >> 6)) {
+                    const int lo = max(bxl - 64 * wx, 0), hi = min(bxh - 64 * wx, 63);
+                    occ_w = __ldg(occ + ((size_t)(m * N + i) * occ_wy + br) * occ_wx + wx) & ((~0ull >> (63 - hi)) & (~0ull << lo));
+                }
+                // ... and it hits L1: a box drifts by a few texels from plane to plane, so the words of plane i + kOccAhead around this
+                // box are fetched now.  (Without it a prompt producer waits a full L2 round trip per stage: -25 % on a white-noise MPI,
+                // where nothing is empty, and no gain where almost everything is.)
+                if (mode == 0 && x0 <= x1 && y0 <= y1) {
+                    constexpr int kOccAhead = 4;
+                    const int ia = min(i + kOccAhead, N - 1);
+                    asm volatile("prefetch.global.L1 [%0];" ::"l"(occ + ((size_t)(m * N + ia) * occ_wy + min(br, occ_wy - 1)) * occ_wx +
+                                                                     min(wx, occ_wx - 1)));
+                }
+            }
             if constexpr (Pacer::kActive) {      // the side job fills the wait for a free stage, a few stores between polls
                 pacer.new_stage();
                 while (!mbar_try_wait(&s_empty[s], ph ^ 1))
@@ -460,6 +513,15 @@ __device__ __forceinline__ void staged_producer(const RenderParams& p, const Tma
                     break;
                 }
                 if (lane == 0) s_vote[s] = 0u;      // published below with the header (the arrive releases both)
+            }
+            if constexpr (kSkip) {
+                // nothing above the threshold in the box; and the plane constants are in the exact-division range, where the
+                // consumers' packed coordinates (their box test) are bit-exact -- the same condition as the class bits
+                if (mode == 0 && pc.fast != 0.0f && !__any_sync(0xffffffffu, occ_w != 0)) {
+                    mode = kModeEmpty;
+                    n_ops = 0;
+                    ++n_empty;
+                }
             }
             if (lane == 0) {
                 StageMeta mt;
@@ -504,6 +566,10 @@ __device__ __forceinline__ void staged_producer(const RenderParams& p, const Tma
                     }
                 }
             }
+        }
+        if constexpr (kSkip) {
+            if (skipped_empty && n_empty && lane == 0)
+                atomicAdd(skipped_empty, (unsigned long long)n_empty * (unsigned long long)(min(kTileW, p.W - px0) * min(kTileH, p.H - py0)));
         }
     }
     if constexpr (Pacer::kActive) pacer.at_end();
@@ -562,13 +628,17 @@ __device__ __forceinline__ void store_tile_pixels(const RenderParams& p, int v, 
 template <bool kFactored>
 using FwdRingFor = typename std::conditional<kFactored && GMPI_FWD_WIDE_FACT != 0, FwdRingWide, FwdRing>::type;
 
-// The staged forward, body of both kernels below.  kCut: early ray termination at T < tau (never with kEmitT); s_vote [kStages]
-// and `skipped` (nullable) as in staged_producer.  With kCut == false the extra arguments are unused and the code is that of the
-// kernel before termination existed.
-template <bool kAlignCorners, bool kEmitT, bool kFactored, bool kCut>
+// The staged forward, body of the kernels below.  kCut: early ray termination at T < tau (never with kEmitT); s_vote [kStages]
+// and `skipped` (nullable) as in staged_producer.  kSkip: empty-space skipping (never with kEmitT); occ and `skipped_empty`
+// (nullable) as in staged_producer.  With kCut == kSkip == false the extra arguments are unused and the code is that of the
+// kernel before either existed.
+template <bool kAlignCorners, bool kEmitT, bool kFactored, bool kCut, bool kSkip = false>
 __device__ __forceinline__ void fwd_staged_body(const RenderParams& p, const TmaMaps& maps, const int tiles_x, const int tiles_y,
-                                                float tau, uint32_t* s_vote, unsigned long long* skipped) {
+                                                float tau, uint32_t* s_vote, unsigned long long* skipped,
+                                                const uint64_t* occ = nullptr, unsigned long long* skipped_empty = nullptr) {
     static_assert(!(kCut && kEmitT), "the training forward saves every T: no termination");
+    static_assert(!(kSkip && kEmitT), "the training forward is exact: no empty-space skipping");
+    constexpr int kModeMask = kSkip ? 7 : 3;      // the header's mode field: 3 bits with kModeEmpty
     extern __shared__ __align__(1024) unsigned char smem_raw[];
     float* s_buf = reinterpret_cast<float*>(smem_raw);   // the ring starts the dynamic segment (1024-byte aligned)
     using Ring = FwdRingFor<kFactored>;
@@ -603,8 +673,10 @@ __device__ __forceinline__ void fwd_staged_body(const RenderParams& p, const Tma
 
     if (warp == kConsWarps) {
         NoPacer np;
-        if constexpr (kCut) staged_producer<kAlignCorners, Ring, kFactored, NoPacer, true>(p, maps, s_buf, s_meta, s_full, s_empty, &s_walk, lane, np,
-                                                                                          s_vote, skipped);
+        if constexpr (kSkip) staged_producer<kAlignCorners, Ring, kFactored, NoPacer, kCut, true>(p, maps, s_buf, s_meta, s_full, s_empty, &s_walk,
+                                                                                                 lane, np, s_vote, skipped, occ, skipped_empty);
+        else if constexpr (kCut) staged_producer<kAlignCorners, Ring, kFactored, NoPacer, true>(p, maps, s_buf, s_meta, s_full, s_empty, &s_walk, lane, np,
+                                                                                               s_vote, skipped);
         else staged_producer<kAlignCorners, Ring, kFactored>(p, maps, s_buf, s_meta, s_full, s_empty, &s_walk, lane, np);
     } else {
         // ================================ consumer warps ================================
@@ -634,7 +706,7 @@ __device__ __forceinline__ void fwd_staged_body(const RenderParams& p, const Tma
                 v_table = v;
             }
             if (py0 + kPairs * warp >= p.H) {      // warp-uniform: no row of this warp is inside the image
-                consumer_idle_tile<kCut>(s_full, s_empty, N, lane, c_stage, c_phase, s_meta);
+                consumer_idle_tile<kCut, kModeMask>(s_full, s_empty, N, lane, c_stage, c_phase, s_meta);
                 continue;
             }
             RayConst rc[kPix];   // scalar copies, only for the generic (rare) body and the epilogue
@@ -686,7 +758,12 @@ __device__ __forceinline__ void fwd_staged_body(const RenderParams& p, const Tma
                 const float* sb = s_buf + s * kRingFloats;
                 const int sel = mt.sel;                  // warp-uniform; the producer already folded mode and plane range in
                 bool done = false;
-                if (warp_fast) {
+                bool empty = false;
+                if constexpr (kSkip) empty = ((sel >> 8) & kModeMask) == kModeEmpty;
+                // (exclusive of the tap chain: testing the empty box in front of the chain instead cost the kSkip kernels a spill)
+                if (empty) {                             // all taps in the empty box: a = 0, nothing to add
+                    if (warp_fast) done = taps_in_box(cc, mt.cx, mt.cy, (sel & 0xff) - 2, mt.rows2);
+                } else if (warp_fast) {
                     if (Ring::kWideFact) {               // factored: two widths, both with bank-aligned row pitches
                         if (sel & (1 << 20)) done = sample_pairs<kWideBW, kAOff>(sb, mt.cx, mt.cy, mt.rows2, cc, T, cr, cg, cb, cws);
                         else if (sel & (1 << 17)) done = sample_pairs<64, kAOff>(sb, mt.cx, mt.cy, mt.rows2, cc, T, cr, cg, cb, cws);
@@ -700,7 +777,8 @@ __device__ __forceinline__ void fwd_staged_body(const RenderParams& p, const Tma
                 }
                 if (!done) {
                     // ---- generic body: per-pixel range / box checks, direct sampling when not staged ----
-                    const int bw = mt.sel & 0xff, mode = (mt.sel >> 8) & 3, bw4 = 4 * bw;
+                    // (kModeEmpty: nothing is staged, mode != 0 sends every pixel to global memory)
+                    const int bw = mt.sel & 0xff, mode = (mt.sel >> 8) & kModeMask, bw4 = 4 * bw;
                     if constexpr (kCut) {
                         if (mode == kModeEnd) {          // the producer cut the tile short: release the stage, go to the epilogue
                             __syncwarp();
@@ -799,6 +877,19 @@ mpi_fwd_cut_kernel(const RenderParams p, const __grid_constant__ TmaMaps maps, c
                    unsigned long long* skipped) {
     __shared__ uint32_t s_vote[kStages];
     fwd_staged_body<kAlignCorners, false, kFactored, true>(p, maps, tiles_x, tiles_y, tau, s_vote, skipped);
+}
+
+// Inference forward with empty-space skipping (see kModeEmpty): occupancy is the map of gmpi_mpi_occupancy for the MPI of p;
+// empty_pixel_planes (nullable) accumulates the pixel-planes of the boxes published empty.  kCut: together with early ray
+// termination (tau, skipped as in mpi_fwd_cut_kernel).  Same ring, same epilogues as mpi_fwd_staged_kernel<kAlignCorners, false,
+// kFactored>.
+template <bool kAlignCorners, bool kFactored, bool kCut>
+__global__ void __launch_bounds__(kStagedThreads, kCtasPerSm)
+mpi_fwd_skip_kernel(const RenderParams p, const __grid_constant__ TmaMaps maps, const int tiles_x, const int tiles_y, const float tau,
+                    unsigned long long* skipped, const uint64_t* __restrict__ occupancy, unsigned long long* empty_pixel_planes) {
+    __shared__ uint32_t s_vote[kStages];
+    fwd_staged_body<kAlignCorners, false, kFactored, kCut, true>(p, maps, tiles_x, tiles_y, tau, s_vote, skipped, occupancy,
+                                                                 empty_pixel_planes);
 }
 
 }  // namespace gmpi

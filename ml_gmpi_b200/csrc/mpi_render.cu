@@ -273,6 +273,58 @@ __global__ void mpi_check_range_scalar_kernel(const float* __restrict__ rgba, si
 }
 
 // ------------------------------------------------------------------------------------------
+// Occupancy map of empty-space skipping (gmpi_mpi_occupancy): one bit per 8x8-texel block of every alpha plane, set iff some
+// alpha of the block has !(|alpha| <= threshold) (NaN is occupied); texels outside the texture do not exist.  One warp per
+// 64-bit word = 8 texel rows x 512 texels: every load of the warp covers 32 * kVec consecutive texels of one row (kVec = 4:
+// float4, rows and strides 16-byte aligned), its ballot has 8 / kVec bits per block; the ballots of the 8 rows are OR-ed, then
+// folded into one bit per block.  A streaming read of the alpha planes alone, 4 bytes per texel-plane.
+// ------------------------------------------------------------------------------------------
+template <int kVec>
+__global__ void __launch_bounds__(256)
+mpi_occupancy_kernel(const float* __restrict__ alpha, long long mpi_stride, long long plane_stride, int N, int Ht, int Wt, int n_wy,
+                     int n_wx, long long n_words, float threshold, uint64_t* __restrict__ occ) {
+    constexpr int kLoads = 512 / (32 * kVec), kLanesPerBlock = 8 / kVec, kBlocksPerLoad = 32 / kLanesPerBlock;
+    const long long word = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    const int lane = threadIdx.x & 31;
+    if (word >= n_words) return;     // warp-uniform
+    const int wx = (int)(word % n_wx);
+    const long long t = word / n_wx;
+    const int wy = (int)(t % n_wy);
+    const long long plane = t / n_wy, m = plane / N, i = plane - m * N;
+    const float* base = alpha + m * mpi_stride + i * plane_stride;
+    uint32_t bal[kLoads];
+#pragma unroll
+    for (int k = 0; k < kLoads; ++k) bal[k] = 0u;
+#pragma unroll
+    for (int r = 0; r < 8; ++r) {
+        const int y = 8 * wy + r;
+        const float* row = base + (long long)y * Wt;
+#pragma unroll
+        for (int k = 0; k < kLoads; ++k) {
+            const int x = 512 * wx + kVec * (32 * k + lane);
+            bool o = false;
+            if (y < Ht && x < Wt) {          // (kVec = 4: Wt % 4 == 0, so the whole float4 is inside the row)
+                if constexpr (kVec == 4) {
+                    const float4 a = __ldcs(reinterpret_cast<const float4*>(row + x));
+                    o = !(fabsf(a.x) <= threshold) || !(fabsf(a.y) <= threshold) || !(fabsf(a.z) <= threshold) || !(fabsf(a.w) <= threshold);
+                } else {
+                    o = !(fabsf(__ldcs(row + x)) <= threshold);
+                }
+            }
+            bal[k] |= __ballot_sync(0xffffffffu, o);
+        }
+    }
+    if (lane != 0) return;
+    uint64_t w = 0;
+#pragma unroll
+    for (int k = 0; k < kLoads; ++k)
+#pragma unroll
+        for (int q = 0; q < kBlocksPerLoad; ++q)
+            if ((bal[k] >> (q * kLanesPerBlock)) & ((1u << kLanesPerBlock) - 1u)) w |= 1ull << (k * kBlocksPerLoad + q);
+    occ[word] = w;
+}
+
+// ------------------------------------------------------------------------------------------
 // Test hook: texel coordinates.
 // ------------------------------------------------------------------------------------------
 template <bool kAlignCorners>
@@ -454,9 +506,26 @@ static cudaError_t launch_fwd_cut(const RenderParams& p, const TmaMaps& maps, in
     kernel<<<grid, kStagedThreads, smem, st>>>(p, maps, tiles_x, tiles_y, p.stop_transmittance, p.skipped);
     return cudaSuccess;
 }
+template <bool AC, bool FAC, bool CUT>
+static cudaError_t launch_fwd_skip(const RenderParams& p, const TmaMaps& maps, int grid, int tiles_x, int tiles_y, const uint64_t* occ,
+                                   unsigned long long* empty, cudaStream_t st) {
+    auto kernel = mpi_fwd_skip_kernel<AC, FAC, CUT>;
+    constexpr size_t smem = FwdRingFor<FAC>::kWideFact ? kStagedSmemWide : kStagedSmem;
+    cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return e;
+    kernel<<<grid, kStagedThreads, smem, st>>>(p, maps, tiles_x, tiles_y, p.stop_transmittance, p.skipped, occ, empty);
+    return cudaSuccess;
+}
+typedef cudaError_t (*SkipLaunch)(const RenderParams&, const TmaMaps&, int, int, int, const uint64_t*, unsigned long long*, cudaStream_t);
+static const SkipLaunch kSkipLaunch[2][2][2] = {     // [align_corners][factored][stop_transmittance > 0]
+    {{launch_fwd_skip<false, false, false>, launch_fwd_skip<false, false, true>},
+     {launch_fwd_skip<false, true, false>, launch_fwd_skip<false, true, true>}},
+    {{launch_fwd_skip<true, false, false>, launch_fwd_skip<true, false, true>},
+     {launch_fwd_skip<true, true, false>, launch_fwd_skip<true, true, true>}}};
 
-// Forward launch for a filled RenderParams.
-static int launch_fwd(RenderParams p, cudaStream_t st) {
+// Forward launch for a filled RenderParams.  occ (nullable): the occupancy map of empty-space skipping, honoured by the staged
+// kernels (the direct kernel renders every plane); `empty` (nullable) accumulates the pixel-planes skipped as empty.
+static int launch_fwd(RenderParams p, cudaStream_t st, const uint64_t* occ = nullptr, unsigned long long* empty = nullptr) {
     int rc = check_params(p, false);
     if (rc) return rc;
     if (!p.flags) return fail(GMPI_ERR_INVALID_ARGUMENT, "null flags pointer");
@@ -486,7 +555,9 @@ static int launch_fwd(RenderParams p, cudaStream_t st) {
             const long n_tiles = (long)tiles_x * tiles_y * p.V;
             const int grid = (int)(n_tiles < (long)sms * kCtasPerSm ? n_tiles : (long)sms * kCtasPerSm);
             cudaError_t e;
-            if (p.stop_transmittance > 0.0f) {      // (check_params: never together with the transmittance output)
+            if (occ) {                              // (gmpi_mpi_render_fwd_skip_ex: never together with the transmittance output)
+                e = kSkipLaunch[ac][fac][p.stop_transmittance > 0.0f](p, maps, grid, tiles_x, tiles_y, occ, empty, st);
+            } else if (p.stop_transmittance > 0.0f) {      // (check_params: never together with the transmittance output)
                 if (fac) e = ac ? launch_fwd_cut<true, true>(p, maps, grid, tiles_x, tiles_y, st) : launch_fwd_cut<false, true>(p, maps, grid, tiles_x, tiles_y, st);
                 else e = ac ? launch_fwd_cut<true, false>(p, maps, grid, tiles_x, tiles_y, st) : launch_fwd_cut<false, false>(p, maps, grid, tiles_x, tiles_y, st);
             } else if (fac) {
@@ -798,6 +869,43 @@ int gmpi_mpi_render_fwd_ex(const gmpi_render_desc* d) {
     int rc = check_desc(d);
     if (rc) return rc;
     return launch_fwd(params_from_desc(d), (cudaStream_t)d->stream);
+}
+
+int gmpi_mpi_render_fwd_skip_ex(const gmpi_render_desc* d, const uint64_t* occupancy, uint64_t* empty_pixel_planes) {
+    int rc = check_desc(d);
+    if (rc) return rc;
+    if (!occupancy) return fail(GMPI_ERR_INVALID_ARGUMENT, "null occupancy map (gmpi_mpi_occupancy builds it)");
+    if (d->transmittance)
+        return fail(GMPI_ERR_INVALID_ARGUMENT, "empty-space skipping with a transmittance buffer: the training forward saves every T "
+                    "and stays exact, skipping is for inference only");
+    return launch_fwd(params_from_desc(d), (cudaStream_t)d->stream, occupancy, reinterpret_cast<unsigned long long*>(empty_pixel_planes));
+}
+
+size_t gmpi_mpi_occupancy_plane_words(int Ht, int Wt) {
+    if (Ht < 1 || Wt < 1) return 0;
+    return (size_t)((Ht + 7) / 8) * (size_t)((Wt + 511) / 512);
+}
+
+int gmpi_mpi_occupancy(const float* alpha, long long mpi_stride, long long plane_stride, int M, int N, int Ht, int Wt, float threshold,
+                       uint64_t* occupancy, void* stream) {
+    if (!alpha || !occupancy) return fail(GMPI_ERR_INVALID_ARGUMENT, "null pointer");
+    if (!(threshold >= 0.0f && threshold < 1.0f))      // (NaN fails both comparisons)
+        return fail(GMPI_ERR_INVALID_ARGUMENT, "occupancy threshold=%g must be in [0, 1)", (double)threshold);
+    if (M < 1 || N < 1 || Ht < 1 || Wt < 1 || mpi_stride < 0 || plane_stride < 0)
+        return fail(GMPI_ERR_INVALID_ARGUMENT, "bad sizes M=%d N=%d Ht=%d Wt=%d", M, N, Ht, Wt);
+    const int n_wy = (Ht + 7) / 8, n_wx = (Wt + 511) / 512;
+    const long long n_words = (long long)M * N * n_wy * n_wx;
+    const long long blocks = (n_words + 7) / 8;      // 8 warps of 256 threads, one word each
+    if (blocks > 0x7fffffffLL) return fail(GMPI_ERR_UNSUPPORTED, "%lld occupancy words exceed one launch", n_words);
+    cudaStream_t st = (cudaStream_t)stream;
+    if (Wt % 4 == 0 && plane_stride % 4 == 0 && mpi_stride % 4 == 0 && ((uintptr_t)alpha & 15) == 0)
+        mpi_occupancy_kernel<4><<<(unsigned)blocks, 256, 0, st>>>(alpha, mpi_stride, plane_stride, N, Ht, Wt, n_wy, n_wx, n_words, threshold,
+                                                                  occupancy);
+    else
+        mpi_occupancy_kernel<1><<<(unsigned)blocks, 256, 0, st>>>(alpha, mpi_stride, plane_stride, N, Ht, Wt, n_wy, n_wx, n_words, threshold,
+                                                                  occupancy);
+    GMPI_CUDA_OK(cudaGetLastError());
+    return GMPI_OK;
 }
 
 int gmpi_mpi_render_bwd_ex(const gmpi_render_desc* d) {

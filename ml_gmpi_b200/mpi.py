@@ -36,7 +36,8 @@ class _RenderFn(torch.autograd.Function):
     The MPI is either expanded (`rgba`) or factored (`rgb`, `alpha`, optional `bg_rgb`); the unused form is None."""
 
     @staticmethod
-    def forward(ctx, rgba, rgb, alpha, bg_rgb, dhw, view2mpi, ray_dir, eye, z_dir, options, flags, view_group, stop_transmittance):
+    def forward(ctx, rgba, rgb, alpha, bg_rgb, dhw, view2mpi, ray_dir, eye, z_dir, options, flags, view_group, stop_transmittance,
+                skip_alpha):
         lib = _lib.load()
         factored = rgba is None
         ref = alpha if factored else rgba
@@ -54,12 +55,13 @@ class _RenderFn(torch.autograd.Function):
         # early ray termination only when no input needs a gradient: with one the render is exact (the backward needs every
         # plane's T), so one MPI object serves the no-grad D step and the G step alike
         tau = float(stop_transmittance) if trans is None else 0.0
+        skip = skip_alpha if trans is None else None         # the same rule for empty-space skipping
         with torch.cuda.device(dev):
             d = _lib.make_desc(options=options, M=M, V=V, N=N, Ht=Ht, Wt=Wt, H=H, W=W, view_group=view_group, rgba=rgba, rgb=rgb,
                                alpha=alpha, bg_rgb=bg_rgb, view2mpi=view2mpi, dhw=dhw, ray_dir=ray_dir, eye=eye, z_dir=z_dir,
                                color=color, depth=depth, transmittance=trans, flags=flags, stream=_stream_ptr(dev),
                                stop_transmittance=tau)
-            _lib.check(lib.gmpi_mpi_render_fwd_ex(ctypes.byref(d)))
+            _render_fwd(lib, d, skip, rgba, alpha, V, H, W)
         ctx.save_for_backward(rgba, rgb, alpha, bg_rgb, dhw, view2mpi, ray_dir, eye, z_dir, trans)
         ctx.options, ctx.view_group = options, view_group
         ctx.set_materialize_grads(False)
@@ -69,7 +71,7 @@ class _RenderFn(torch.autograd.Function):
     @torch.autograd.function.once_differentiable     # raw kernels: a double backward (create_graph=True) must raise, not
     def backward(ctx, g_color, g_depth):             # silently treat the result as constant (the reference's R1 only differentiates D)
         rgba, rgb, alpha, bg_rgb, dhw, view2mpi, ray_dir, eye, z_dir, trans = ctx.saved_tensors
-        none = (None,) * 13
+        none = (None,) * 14
         if not any(ctx.needs_input_grad[:4]):
             return none
         lib = _lib.load()
@@ -98,7 +100,7 @@ class _RenderFn(torch.autograd.Function):
                                ray_dir=ray_dir, eye=eye, z_dir=z_dir, transmittance=trans, g_color=g_color, g_depth=g_depth,
                                g_rgba=g_rgba, g_rgb=g_rgb, g_bg_rgb=g_bg, g_alpha=g_alpha, stream=_stream_ptr(dev))
             _lib.check(lib.gmpi_mpi_render_bwd_ex(ctypes.byref(d)))
-        return (g_rgba, g_rgb, g_alpha, g_bg) + (None,) * 9
+        return (g_rgba, g_rgb, g_alpha, g_bg) + (None,) * 10
 
 
 _warned_direct = set()
@@ -131,15 +133,64 @@ def _check_stop(stop_transmittance) -> float:
     return tau
 
 
+def _check_skip(skip_alpha) -> Optional[float]:
+    if skip_alpha is None:
+        return None
+    eps = float(skip_alpha)
+    if not 0.0 <= eps < 1.0:
+        raise ValueError(f"skip_alpha must be None or in [0, 1), got {skip_alpha}")
+    return eps
+
+
+def occupancy_map(threshold: float, *, rgba: Optional[torch.Tensor] = None, alpha: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """Occupancy map of empty-space skipping (gmpi_mpi_occupancy), built on the current stream from the expanded stack rgba
+    [M,N,4,Ht,Wt] (its channel 3, no copy) or the factored alpha [M,N,1,Ht,Wt] (contiguous fp32 CUDA tensors): one bit per 8x8-texel
+    block of every plane, set iff some alpha of the block exceeds `threshold` in magnitude (or is NaN).  Returned as an int64 tensor
+    [M, N, ceil(Ht/8), ceil(Wt/512)] holding the uint64 words of the C layout."""
+    ref = alpha if rgba is None else rgba
+    M, N = ref.shape[0], ref.shape[1]
+    Ht, Wt = ref.shape[-2:]
+    tex = Ht * Wt
+    occ = torch.empty((M, N, (Ht + 7) // 8, (Wt + 511) // 512), dtype=torch.int64, device=ref.device)
+    if rgba is not None:
+        ptr, plane_stride = rgba.data_ptr() + 4 * 3 * tex, 4 * tex          # channel 3 of every plane
+    else:
+        ptr, plane_stride = alpha.data_ptr(), tex
+    with torch.cuda.device(ref.device):
+        _lib.check(_lib.load().gmpi_mpi_occupancy(ptr, N * plane_stride, plane_stride, M, N, Ht, Wt, float(threshold), occ.data_ptr(),
+                                                  _stream_ptr(ref.device)))
+    return occ
+
+
+def _render_fwd(lib, d, skip_alpha, rgba, alpha, V, H, W, empty=None):
+    """The forward of descriptor d: gmpi_mpi_render_fwd_ex, or -- skip_alpha set and the shapes take the staged kernel -- the
+    skipping forward on an occupancy map built for this call (the direct kernel would ignore it: no map then).  `empty` (nullable
+    int64 tensor of one element) receives the skipped pixel-planes.  Call on the render's device."""
+    if skip_alpha is not None:
+        ref = alpha if rgba is None else rgba
+        N, (Ht, Wt) = ref.shape[1], ref.shape[-2:]
+        if lib.gmpi_mpi_render_fwd_plan(V, N, Ht, Wt, H, W, ref.data_ptr(), None) == _lib.PLAN_STAGED:
+            occ = occupancy_map(skip_alpha, rgba=rgba, alpha=alpha)
+            _lib.check(lib.gmpi_mpi_render_fwd_skip_ex(ctypes.byref(d), occ.data_ptr(), None if empty is None else empty.data_ptr()))
+            return
+    _lib.check(lib.gmpi_mpi_render_fwd_ex(ctypes.byref(d)))
+
+
 def render_views(rgba, dhw, view2mpi, ray_dir, eye, z_dir, *, align_corners=True, check_last_plane=False,
-                 color_minus1_1=False, flags: Optional[torch.Tensor] = None, view_group: int = 1, stop_transmittance: float = 0.0):
+                 color_minus1_1=False, flags: Optional[torch.Tensor] = None, view_group: int = 1, stop_transmittance: float = 0.0,
+                 skip_alpha: Optional[float] = None):
     """Functional form on packed tensors (no list handling, no host sync).
     rgba [M,N,4,Ht,Wt], dhw [M,N,3], view2mpi [V] int32, ray_dir [V,3,H,W], eye/z_dir [V,3].
     Returns (color [V,3,H,W], depth [V,1,H,W]); `flags` (uint32 tensor of 1, int32 storage) is OR-ed into.
     view_group > 1: every view_group consecutive views share one MPI (tile-order hint: L2 reuse, see the C header).
     stop_transmittance = tau in (0, 1): early ray termination when no input needs a gradient -- a pixel may drop the planes
     behind the point where its transmittance fell below tau, so every output is within tau * max(value) below the exact one
-    (the contract in include/gmpi_mpi_render.h).  0 (default): exact.  Ignored (exact render) when rgba requires grad."""
+    (the contract in include/gmpi_mpi_render.h).  0 (default): exact.  Ignored (exact render) when rgba requires grad.
+    skip_alpha = eps: empty-space skipping when no input needs a gradient -- the call builds an occupancy map of the MPI (one
+    streaming read of alpha) and the kernel skips the (64x30 tile, plane) pairs whose alpha is within eps of 0 under the whole
+    tile.  0.0 skips only exactly transparent space and is bit-identical to the exact render; eps in (0, 1) moves every output by
+    at most N * eps * max(value) (colour and alpha in [0, 1]).  None (default): off.  Ignored (exact render) when rgba requires
+    grad, like stop_transmittance."""
     if not rgba.is_cuda:
         raise RuntimeError("ml_gmpi_b200 renders on CUDA devices only (no CPU fallback); got a CPU tensor")
     if flags is None:
@@ -147,17 +198,18 @@ def render_views(rgba, dhw, view2mpi, ray_dir, eye, z_dir, *, align_corners=True
     _warn_if_direct(rgba, ray_dir.shape[0], ray_dir.shape[2], ray_dir.shape[3])
     return _RenderFn.apply(_as_f32c(rgba), None, None, None, _as_f32c(dhw), view2mpi, _as_f32c(ray_dir), _as_f32c(eye), _as_f32c(z_dir),
                            _options(align_corners, check_last_plane, color_minus1_1), flags, int(view_group),
-                           _check_stop(stop_transmittance))
+                           _check_stop(stop_transmittance), _check_skip(skip_alpha))
 
 
 def render_views_factored(rgb, alpha, dhw, view2mpi, ray_dir, eye, z_dir, *, bg_rgb=None, align_corners=True,
                           check_last_plane=False, color_minus1_1=False, flags: Optional[torch.Tensor] = None, view_group: int = 1,
-                          stop_transmittance: float = 0.0):
+                          stop_transmittance: float = 0.0, skip_alpha: Optional[float] = None):
     """The same render from the generator's FACTORED output (networks_cond_on_pos_enc.py:950-975,984): one colour image
     rgb [M,3,Ht,Wt] shared by all planes (bg_rgb [M,3,Ht,Wt]: the last plane's own colour under torgba_sep_background) and
     alpha [M,N,1,Ht,Wt] -- what the reference expands to [M,N,4,Ht,Wt] (and copies per view, train.py:553-558,733-738) before
     rendering.  Output identical to render_views on the expanded stack, 4x fewer HBM bytes; differentiable w.r.t. rgb, alpha
-    and bg_rgb (d/d rgb is the sum over the planes that share it).  stop_transmittance: as in render_views."""
+    and bg_rgb (d/d rgb is the sum over the planes that share it).  stop_transmittance, skip_alpha (the map is built from
+    `alpha`): as in render_views."""
     if not alpha.is_cuda:
         raise RuntimeError("ml_gmpi_b200 renders on CUDA devices only (no CPU fallback); got a CPU tensor")
     assert rgb.ndim == 4 and rgb.shape[1] == 3 and alpha.ndim == 5 and alpha.shape[2] == 1 and rgb.shape[0] == alpha.shape[0] \
@@ -168,7 +220,7 @@ def render_views_factored(rgb, alpha, dhw, view2mpi, ray_dir, eye, z_dir, *, bg_
     _warn_if_direct(alpha, ray_dir.shape[0], ray_dir.shape[2], ray_dir.shape[3])
     return _RenderFn.apply(None, _as_f32c(rgb), _as_f32c(alpha), None if bg_rgb is None else _as_f32c(bg_rgb), _as_f32c(dhw), view2mpi,
                            _as_f32c(ray_dir), _as_f32c(eye), _as_f32c(z_dir), _options(align_corners, check_last_plane, color_minus1_1),
-                           flags, int(view_group), _check_stop(stop_transmittance))
+                           flags, int(view_group), _check_stop(stop_transmittance), _check_skip(skip_alpha))
 
 
 def expand_factored(rgb, alpha, bg_rgb=None):
@@ -184,13 +236,16 @@ def expand_factored(rgb, alpha, bg_rgb=None):
 def render_frames(*, dhw, view2mpi, rgba=None, rgb=None, alpha=None, bg_rgb=None, ray_dir=None, eye=None, z_dir=None, cam=None,
                   align_corners=True, check_last_plane=False, video: Optional[dict] = None, u8_round=False,
                   flags: Optional[torch.Tensor] = None, view_group: int = 1, H: Optional[int] = None, W: Optional[int] = None,
-                  stop_transmittance: float = 0.0, skipped: Optional[torch.Tensor] = None):
+                  stop_transmittance: float = 0.0, skipped: Optional[torch.Tensor] = None, skip_alpha: Optional[float] = None,
+                  skipped_empty: Optional[torch.Tensor] = None):
     """Inference-only render with the opt-in fast paths of the C ABI (no autograd):
       cam [V,16]     rays generated in the kernel from the pinhole camera (see camera.cam_params) instead of ray_dir/eye/z_dir;
       video={"near": ray_start, "far": ray_end, "depth": True}   uint8 HWC frames as render_video.py:118-126 builds them:
                      returns (rgb_u8 [V,H,W,3], depth_u8 [V,H,W,1] or None); otherwise (color in [-1,1], depth) fp32.
       stop_transmittance = tau in (0, 1)   early ray termination (see render_views; the [-1,1] colour moves by up to 2 tau);
       skipped        int64 CUDA tensor of one element: the number of pixel-planes not composited is added to it.
+      skip_alpha = eps in [0, 1)   empty-space skipping (see render_views; one occupancy map per call, for all its views);
+      skipped_empty  int64 CUDA tensor of one element: the number of pixel-planes skipped as empty is added to it.
     """
     ref = alpha if rgba is None else rgba
     if not ref.is_cuda:
@@ -209,8 +264,10 @@ def render_frames(*, dhw, view2mpi, rgba=None, rgb=None, alpha=None, bg_rgb=None
     if flags is None:
         flags = torch.zeros(1, dtype=torch.int32, device=dev)
     tau = _check_stop(stop_transmittance)
-    if skipped is not None and not (skipped.is_cuda and skipped.dtype == torch.int64 and skipped.numel() == 1 and skipped.is_contiguous()):
-        raise ValueError("skipped must be a contiguous int64 CUDA tensor of one element")
+    eps = _check_skip(skip_alpha)
+    for name, t in (("skipped", skipped), ("skipped_empty", skipped_empty)):
+        if t is not None and not (t.is_cuda and t.dtype == torch.int64 and t.numel() == 1 and t.is_contiguous()):
+            raise ValueError(f"{name} must be a contiguous int64 CUDA tensor of one element")
     color = depth = v_rgb = v_depth = None
     near = rng = 0.0
     if video is not None:
@@ -229,7 +286,7 @@ def render_frames(*, dhw, view2mpi, rgba=None, rgb=None, alpha=None, bg_rgb=None
                            bg_rgb=keep[3], view2mpi=view2mpi, dhw=keep[4], ray_dir=ray_dir, eye=eye, z_dir=z_dir, cam=cam, color=color,
                            depth=depth, video_rgb=v_rgb, video_depth=v_depth, flags=flags, stream=_stream_ptr(dev),
                            stop_transmittance=tau, skipped_pixel_planes=skipped)
-        _lib.check(lib.gmpi_mpi_render_fwd_ex(ctypes.byref(d)))
+        _render_fwd(lib, d, eps, keep[0], keep[2], V, H, W, skipped_empty)
     return (v_rgb, v_depth) if video is not None else (color, depth)
 
 
@@ -251,6 +308,8 @@ class MPI(nn.Module):
          "off"   like "defer" without the last-plane check.
     `stop_transmittance` = tau in (0, 1): early ray termination of renders where no input needs a gradient (see render_views);
     renders with a gradient stay exact.  0 (default): exact.
+    `skip_alpha` (attribute, not a constructor parameter): empty-space skipping threshold of the same renders (see render_views).
+    None (default): off; 0.0: exactly transparent space only (bit-identical output).
     """
 
     def __init__(self, align_corners=True, validate: str = "full", stop_transmittance: float = 0.0):
@@ -259,8 +318,17 @@ class MPI(nn.Module):
         self._align_corners = align_corners
         self.validate = validate
         self.stop_transmittance = _check_stop(stop_transmittance)
+        self._skip_alpha = None
         self._flags = None
         self._flag_ctx = None
+
+    @property
+    def skip_alpha(self) -> Optional[float]:
+        return self._skip_alpha
+
+    @skip_alpha.setter
+    def skip_alpha(self, value):
+        self._skip_alpha = _check_skip(value)      # ValueError outside [0, 1)
 
     # -- reference: MPI.check_shapes, mpi.py:161-216 (shape part; the alpha range is checked on the device)
     def check_shapes(self, *, batch_rgba, batch_dhw, batch_ray_dir, batch_eye_pos, batch_z_dir, separate_background):
@@ -324,7 +392,7 @@ class MPI(nn.Module):
                                     align_corners=self._align_corners,
                                     check_last_plane=bool(assert_not_out_of_last_plane) and self.validate != "off",
                                     flags=flags, view_group=self.view_group_of(batch_ray_dir),
-                                    stop_transmittance=self.stop_transmittance)
+                                    stop_transmittance=self.stop_transmittance, skip_alpha=self.skip_alpha)
         self._flags = flags
         self._flag_ctx = (batch_dhw, eye, c2w_mat, sphere_c)
         if self.validate == "full":

@@ -35,32 +35,34 @@ def sweep_angles(n_views: int = 100, horizontal: bool = True, mean: float = 0.0)
     return [float(a) + mean for a in np.linspace(half, -half, n_views).tolist()]
 
 
-def _default_video_render(rgba, dhw, c2w, img_size, fov_deg, near, far, fast_rays, factored, stop_transmittance=0.0):
+def _default_video_render(rgba, dhw, c2w, img_size, fov_deg, near, far, fast_rays, factored, stop_transmittance=0.0, skip_alpha=None):
     from .mpi import render_frames
     dev = dhw.device
     V = c2w.shape[0]
     v2m = torch.zeros(V, dtype=torch.int32, device=dev)
     kw = dict(rgb=factored[0], alpha=factored[1], bg_rgb=factored[2]) if factored is not None else dict(rgba=rgba)
+    kw.update(stop_transmittance=stop_transmittance, skip_alpha=skip_alpha)     # one call: one occupancy map for the sweep
     if fast_rays:
         cam = cam_params(c2w.to(dev), focal_from_fov(fov_deg, img_size), img_size, img_size)
         return render_frames(dhw=dhw, view2mpi=v2m, cam=cam, H=img_size, W=img_size, video={"near": near, "far": far},
-                             check_last_plane=True, view_group=V, stop_transmittance=stop_transmittance, **kw)
+                             check_last_plane=True, view_group=V, **kw)
     ray_dir, eye, z_dir = PinholeCamera.from_fov(fov_deg, img_size, img_size).generate_rays(c2w.to(dev))
     return render_frames(dhw=dhw, view2mpi=v2m, ray_dir=ray_dir, eye=eye, z_dir=z_dir, video={"near": near, "far": far},
-                         check_last_plane=True, view_group=V, stop_transmittance=stop_transmittance, **kw)
+                         check_last_plane=True, view_group=V, **kw)
 
 
 def render_video_frames(mpi_rgba: Optional[torch.Tensor], dhw: torch.Tensor, angles: Sequence[float], *, img_size: int, fov_deg: float,
                         ray_start: float, ray_end: float, sphere_center, sphere_r: float, horizontal: bool = True,
                         other_angle: float = 0.0, fast_rays: bool = False, factored: Optional[Tuple] = None,
                         rank: int = 0, world: int = 1, gather: bool = True, render_fn: Optional[Callable] = None,
-                        stop_transmittance: float = 0.0):
+                        stop_transmittance: float = 0.0, skip_alpha: Optional[float] = None):
     """All `angles` (yaw sweep if `horizontal`, else pitch sweep; the other angle fixed) of ONE MPI ([1,N,4,T,T], or
     factored=(rgb [1,3,T,T], alpha [1,N,1,T,T], bg_rgb or None)) as uint8 frames.
     Returns (img [V,H,W,3] uint8, depth [V,H,W,1] uint8) as CPU tensors: all V views when `gather` (every rank), else this rank's
     slice [lo, hi) of shard_range(V, rank, world).
     stop_transmittance: early ray termination of the render (see mpi.render_views); handed to `render_fn` as a keyword
-    argument when it is not 0, so render functions without the parameter keep working for exact renders."""
+    argument when it is not 0, so render functions without the parameter keep working for exact renders.  skip_alpha:
+    empty-space skipping (see mpi.render_views), likewise handed on only when it is not None."""
     V = len(angles)
     lo, hi = shard_range(V, rank, world)
     a = torch.tensor(list(angles[lo:hi]), dtype=torch.float32).reshape(-1, 1)
@@ -70,6 +72,8 @@ def render_video_frames(mpi_rgba: Optional[torch.Tensor], dhw: torch.Tensor, ang
     fn = render_fn or _default_video_render
     if hi > lo:
         extra = {"stop_transmittance": float(stop_transmittance)} if stop_transmittance else {}
+        if skip_alpha is not None:
+            extra["skip_alpha"] = float(skip_alpha)
         img, depth = fn(mpi_rgba, dhw, c2w, img_size, fov_deg, ray_start, ray_end, fast_rays, factored, **extra)
     else:
         dev = dhw.device

@@ -79,14 +79,21 @@ def surface_alpha(n_mpi, n_planes, tex, *, device="cpu", front=0.2, back=0.75, b
 
 
 def make_workload(kind, *, n_planes, tex, img, n_mpi, views_per_mpi=1, seed=1234, device="cpu", yaws=None, pitches=None) -> Case:
-    """Early-ray-termination workloads, random colours and last plane alpha = 1 in all three:
+    """Early-ray-termination and empty-space-skipping workloads, random colours and last plane alpha = 1 in all of them:
       "noise"   white-noise alpha (make_case(last_alpha_one=True)): T falls below 2^-24 after a few dozen planes everywhere;
       "surface" surface_alpha: only tiles inside the head can terminate;
-      "empty"   alpha = 0 except the last plane: nothing can be skipped (the cost of the termination test alone)."""
+      "empty"   alpha = 0 except the last plane: nothing can be skipped (the cost of the termination test alone);
+      "haze"    "surface" with alpha uniform in [0, 2^-12) where it is 0 there: empty-space skipping at threshold 0 finds nothing
+                to skip, at threshold 2^-12 everything in front of and around the head."""
     case = make_case(n_planes=n_planes, tex=tex, img=img, n_mpi=n_mpi, views_per_mpi=views_per_mpi, seed=seed, device=device,
                      last_alpha_one=True, yaws=yaws, pitches=pitches)
-    if kind == "surface":
+    if kind in ("surface", "haze"):
         case.rgba[:, :, 3:] = surface_alpha(n_mpi, n_planes, tex, device=device)
+        if kind == "haze":
+            gen = torch.Generator(device=device).manual_seed(seed + 1)
+            a = case.rgba[:, :, 3]
+            haze = torch.rand(a.shape, generator=gen, device=device, dtype=torch.float32) * 2.0 ** -12
+            case.rgba[:, :, 3] = torch.where(a == 0, haze, a)
     elif kind == "empty":
         case.rgba[:, :, 3] = 0.0
         case.rgba[:, -1, 3] = 1.0
